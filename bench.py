@@ -8,11 +8,18 @@ over the whole batch.
 
   python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  (CPU restatement of the reference)
+  python bench.py ... --dump-outputs DIR                   (also write the last step's results)
 
 Prints ONE JSON line on rank 0.  `value` is device-resident throughput (inputs already in
 HBM), `e2e` goes through the reference-facing C-ABI call with pinned HOST buffers (H2D and
 D2H inside the timed region).  Weak scaling: every rank owns its own 100k-problem shard, no
 data-path collective (SURVEY.md §8(e)).
+
+--dump-outputs DIR writes what the device-resident path returned in its last timed step, so
+that two builds run with the same arguments (hence the same inputs) can be compared output
+for output: eigenvalues.npy [problems][N][2] (real, imaginary parts), info.npy [problems] and
+problem_index.npy [problems] (index of each problem in the batch), all float64.  Above 64 MiB
+in all, a fixed seeded sample of the problems is written.  With N > 1 GPUs, rank 0's shard.
 """
 from __future__ import annotations
 
@@ -27,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ next to the sources
 
 N_ORDER = 32
 PERIOD = 8
@@ -393,6 +401,29 @@ def multi_device_handle_leg(psd_b200, L, torch, world, B, n, p):
     return out
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+NPY_HEADER_BYTES = 4096  # allowance per file, far above numpy's actual header size
+
+
+def dump_outputs(out_dir, E, I):
+    """Write the device-resident path's results E [B][n][2] and I [B] (see --dump-outputs): every
+    problem when they fit DUMP_LIMIT_BYTES, else a seeded sample of problems in batch order."""
+    import numpy as np
+    import torch
+    B = E.shape[0]
+    per_problem = (E[0].numel() + 2) * 8   # eigenvalues, info and index, as float64
+    budget = DUMP_LIMIT_BYTES - 3 * NPY_HEADER_BYTES
+    if B * per_problem <= budget:
+        idx = np.arange(B)
+    else:
+        idx = np.sort(np.random.default_rng(SEED).choice(B, budget // per_problem, replace=False))
+    sel = torch.from_numpy(idx).to(E.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "eigenvalues.npy"), E[sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "info.npy"), I[sel].cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "problem_index.npy"), idx.astype(np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -466,6 +497,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     kt = h.kernel_times()
     h.set_profiling(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dE, dI)
     kernel_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = evs[0][0].elapsed_time(evs[-1][1])
     total_ms = max_over_ranks(total_ms)
@@ -479,7 +512,7 @@ def run_ours(args):
             h.ptr, n, p, B, 0, 0, 0, 30, C.c_void_p(hA.data_ptr()), None,
             C.c_void_p(hE.data_ptr()), C.c_void_p(hI.data_ptr())))
 
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     step_e2e()  # warm-up (allocates the handle's device buffers)
     barrier()
     t0 = time.perf_counter()
@@ -626,7 +659,13 @@ def main():
     ap.add_argument("--batch", type=int, default=100000, help="problems per GPU per step")
     ap.add_argument("--no-large", dest="no_large", action="store_true",
                     help="skip the large-N (p=4, N=4096) block of the N=1 line")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     try:

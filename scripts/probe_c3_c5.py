@@ -1,5 +1,6 @@
 import sys, time, os
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+ROOT=os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0,ROOT); sys.path.insert(0,os.path.join(ROOT,'tests'))
 import numpy as np, psd_b200, psd_rng
 h=psd_b200.Handle([0])
 S=[k%2 for k in range(10)]
