@@ -363,27 +363,56 @@ int launch_real_eig32(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t stre
       R.A = dA + (size_t)off * p * nn;
       R.packed_out = aux.dPacked;
       R.counter = aux.dCounter;
-      // p >= 2: two warps per problem (left / right half of every reflector step on two schedulers)
-      const bool pair = p >= 2 && !dbg_env("PSD_NO_HESS_PAIR");
+      // p >= 2: two warps per problem (rphess_pair32_kernel_t), or, where it is faster, a chain warp
+      // that runs the reflector chain up to p-2 steps ahead of two warps applying the left and right
+      // updates (rphess_ahead32_kernel_t).  The chain-ahead kernel needs p >= 7 to run far enough
+      // ahead (measured slower at p = 3..6), and its 168-register warps must not leave fewer
+      // problems resident per SM than the two-warp kernel (measured slower at N = 17, p = 8, where
+      // registers hold it to 4 problems per SM against 12).  p = 1 keeps one warp per problem.
       const bool special = n == 32 && p == 8 && !dbg_env("PSD_NO_SPECIAL");
-      void (*hk)(psd::Hess32Params) =
-          pair ? (special ? psd::rphess_pair32_kernel_t<32, 8> : psd::rphess_pair32_kernel_t<0, 0>)
-               : (special ? psd::rphess_warp32_kernel_t<32, 8> : psd::rphess_warp32_kernel_t<0, 0>);
-      const int wpp = pair ? 2 : 1;  // warps per problem
-      cudaFuncAttributes fh;
-      PSD_CUDA(cudaFuncGetAttributes(&fh, hk));
-      const size_t max_dyn1 = (size_t)optin - fh.sharedSizeBytes;
-      const size_t per1 = (size_t)p * R.ld * n * sizeof(double);
-      int wpb1 = (int)std::min<size_t>(8, max_dyn1 / per1);
-      if (wpb1 < 1) return fail(PSD_ERR_UNSUPPORTED, "problem does not fit in shared memory");
-      const size_t smem1 = (size_t)wpb1 * per1;
-      PSD_CUDA(cudaFuncSetAttribute(hk, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)max_dyn1));
-      int occ1 = 0;
-      PSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ1, hk, wpb1 * wpp * 32, smem1));
-      if (occ1 < 1) return fail(PSD_ERR_UNSUPPORTED, "reduction kernel does not fit on an SM");
+      struct Shape {
+        void (*k)(psd::Hess32Params);
+        int wpp, wpb, occ;
+        size_t smem;
+      };
+      const size_t staged = (size_t)p * R.ld * n * sizeof(double);
+      auto shape = [&](void (*k)(psd::Hess32Params), int wpp, size_t per, Shape& sh) -> int {
+        cudaFuncAttributes fh;
+        PSD_CUDA(cudaFuncGetAttributes(&fh, k));
+        const size_t max_dyn = (size_t)optin - fh.sharedSizeBytes;
+        sh.k = k;
+        sh.wpp = wpp;
+        sh.wpb = (int)std::min<size_t>(std::min(8, fh.maxThreadsPerBlock / (32 * wpp)), max_dyn / per);
+        sh.occ = 0;
+        if (sh.wpb < 1) return PSD_OK;
+        sh.smem = (size_t)sh.wpb * per;
+        PSD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_dyn));
+        PSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sh.occ, k, sh.wpb * wpp * 32, sh.smem));
+        return PSD_OK;
+      };
+      Shape hs;
+      if (p == 1) {
+        if ((e = shape(special ? psd::rphess_warp32_kernel_t<32, 8> : psd::rphess_warp32_kernel_t<0, 0>, 1, staged, hs)))
+          return e;
+      } else {
+        if ((e = shape(psd::rphess_pair32_kernel_t<0, 0>, 2, staged, hs))) return e;
+        if (p >= 7) {
+          Shape as;
+          if ((e = shape(special ? psd::rphess_ahead32_kernel_t<32, 8> : psd::rphess_ahead32_kernel_t<0, 0>,
+                         psd::AHEAD_WARPS, psd::ahead_problem_doubles(n, p, R.ld) * sizeof(double), as)))
+            return e;
+          if (as.occ > 0 && as.wpb * as.occ >= hs.wpb * hs.occ) hs = as;
+        }
+      }
+      if (hs.occ < 1) return fail(PSD_ERR_UNSUPPORTED, "reduction kernel does not fit on an SM");
+      const int wpb1 = hs.wpb, wpp = hs.wpp, occ1 = hs.occ;
+      const size_t smem1 = hs.smem;
+      void (*hk)(psd::Hess32Params) = hs.k;
       const long long ctas1 = (nb + wpb1 - 1) / wpb1;
       const int grid1 = (int)std::max(1LL, std::min((long long)occ1 * dev.sm_count, ctas1));
+      if (dbg_env("PSD_GEN_PROF"))
+        fprintf(stderr, "[psd hess32] %d warps/problem, %d problems/CTA x %d CTAs/SM, %zu B smem/CTA\n", wpp, wpb1,
+                occ1, smem1);
       {
         ScopedKernelTimer tm(h, dev, stream, 0);
         hk<<<grid1, wpb1 * wpp * 32, smem1, stream>>>(R);
