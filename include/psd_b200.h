@@ -85,6 +85,9 @@ int psd_handle_device_count(psd_handle_t handle);
  * one problem at a time on the whole GPU (DESIGN.md section 9); results of this path are not
  * bit-for-bit reproducible from run to run (floating-point atomics in the blocked reduction,
  * timing-dependent choice between equally valid shift sets), all acceptance predicates hold.
+ * maxitfac bounds this iteration too: its rounds are capped at (256 + 100 n / D) maxitfac / 30
+ * (D = 32..16 rows per round, by period); a problem that reaches the cap is finished by the
+ * single-bulge team iteration with the same maxitfac.
  * ------------------------------------------------------------------------------------- */
 int psd_rpschur_batched(psd_handle_t handle, int n, int p, int64_t batch, int orientation,
                         int wantT, int wantZ, int maxitfac, double* A, double* Z, double* eig,

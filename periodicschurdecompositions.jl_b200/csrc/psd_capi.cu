@@ -650,12 +650,12 @@ int launch_real_large(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t stre
         h->ms_last = res;
       }
       __atomic_fetch_add(&h->stats[0], (int64_t)res.launches, __ATOMIC_RELAXED);
-      if (res.status == 0) {
+      if (res.status != 1) {  // 0 finished; 2 failed, info set
         if (scaled) PSD_CUDA(psd::ms::postscale(stream, aux.ms, n, p, Ap, rc.wantT, dEig + (size_t)b * 2 * n));
         continue;
       }
-      // no convergence: the factors are still Hessenberg-triangular with Z accumulated, let the
-      // single-bulge team kernel finish this problem
+      // no convergence: the iteration drained its bulges, so the factors are still
+      // Hessenberg-triangular with Z accumulated; the single-bulge team kernel finishes this problem
     }
     if (batch == 1) {
       team_needed = true;

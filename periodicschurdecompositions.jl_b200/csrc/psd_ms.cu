@@ -587,7 +587,7 @@ cudaError_t iterate(cudaStream_t caller, int sm_count, Workspace* ws, int n, int
   const Geom g = be.g;
   MS_CHECK(grow(ws->dU, ws->capU, (size_t)2 * p * n * g.W * sizeof(double)));
   DriverConfig cfg;
-  cfg.n = n; cfg.p = p; cfg.wantT = wantT; cfg.wantZ = be.wantZ;
+  cfg.n = n; cfg.p = p; cfg.wantT = wantT; cfg.wantZ = be.wantZ; cfg.maxitfac = be.maxitfac;
   // Shift window: 12 x 12 (six shift pairs per set).  Larger windows give better Ritz values, but
   // the one-CTA computation takes longer (64 x 64: 14 ms, during which the first launch of every
   // round on the main stream was measured to start 100 - 140 us late), and with dozens of packets
@@ -655,6 +655,12 @@ cudaError_t iterate(cudaStream_t caller, int sm_count, Workspace* ws, int n, int
     cudaStreamWaitEvent(caller, ws->evOut, 0);
   }
   if (!be.ok()) return be.err;
+  if (status == 2) {
+    // the drain did not end: the factors may hold bulges, so no fallback may run on them
+    const int level = n;
+    MS_CHECK(cudaMemcpyAsync(dInfo, &level, sizeof(int), cudaMemcpyHostToDevice, st));
+    MS_CHECK(cudaStreamSynchronize(st));
+  }
   // windows whose packet had no bulge left (identity U_j): their updates were skipped
   int idle_windows = 0;
   cudaMemcpyAsync(&idle_windows, ws->dCtl + kCtlMisc + 6, sizeof(int), cudaMemcpyDeviceToHost, st);

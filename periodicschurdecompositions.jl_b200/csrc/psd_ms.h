@@ -27,7 +27,8 @@ Workspace* ws_create();
 void ws_destroy(Workspace* ws);
 
 struct Result {
-  int status = 0;        // 0 finished, 1 no convergence (valid Hessenberg-triangular state left)
+  int status = 0;        // 0 finished, 1 no convergence (valid Hessenberg-triangular state left),
+                         // 2 failed (*dInfo = n; the state is not usable for a fallback)
   int sweeps = 0;
   long long rounds = 0, windows = 0, shift_pairs = 0;
   int exceptional = 0, final_blocks = 0;
@@ -49,7 +50,8 @@ cudaError_t postscale(cudaStream_t st, Workspace* ws, int n, int p, double* cons
 
 // Periodic QR iteration on Hessenberg-triangular factors H[0..p-1] (internal rightwards order,
 // column-major, ld = n), Z[j] preset to the Q_j of the reduction (or nullptr).  Eigenvalues to
-// dEig[n][2]; *dInfo gets max(*dInfo, failing level).  Synchronises the stream internally.
+// dEig[n][2]; *dInfo gets max(*dInfo, failing level).  maxitfac (<= 0: 30) scales the cap on the
+// rounds of the iteration.  Synchronises the stream internally.
 cudaError_t iterate(cudaStream_t st, int sm_count, Workspace* ws, int n, int p, double* const* H,
                     double* const* Z, int wantT, int wantZ, int maxitfac, double* dEig, int* dInfo,
                     int profile, Result* res);

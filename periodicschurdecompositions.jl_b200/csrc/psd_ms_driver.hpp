@@ -58,7 +58,8 @@ struct DriverConfig {
   int lag = 3;          // rounds between a scan and the plan that uses it
   int shift_blocks = 1; // consecutive shift sets come from this many different trailing diagonal blocks
   int scan_every = 1;   // the subdiagonal is scanned after every scan_every-th round
-  long long max_rounds = 0;  // 0: 64 + 40 n / D
+  long long max_rounds = 0;  // 0: (256 + 100 n / D) maxitfac / 30
+  int maxitfac = 30;    // the caller's iteration budget factor (<= 0: 30), scales the round cap
   int max_blocks = 4;   // active diagonal blocks worked on concurrently (1: only the lowest, like the reference)
   int new_block_delay = 4;  // rounds between the first shift request of a new block and its first packet
                             // (its own shift set is then normally complete; measured in profiles/r2_large_n_tuning.md)
@@ -76,6 +77,7 @@ struct Packet {
   int nbul, pair0, npairs, pair_off;
   int ilo, ihi;  // active block when the packet was introduced
   int fin_s;     // position at which the packet was first seen in finished territory (-1: not yet)
+  WinDesc last;  // its window of the latest round it took part in (hops > 0)
 };
 
 // Shift supply and stagnation counters of one active block.
@@ -90,12 +92,27 @@ struct BlockCtl {
 };
 
 // status: 0 = reduced to blocks of order <= W and finished; 1 = no convergence (the factors are
-// still a valid Hessenberg-triangular form with Z accumulated; the caller may fall back).
+// still a valid Hessenberg-triangular form with Z accumulated; the caller may fall back); 2 = the
+// drain before status 1 did not end within its bound (factors unusable; the caller reports failure).
+//
+// Giving up (round cap, stagnation, or two windows of one round that would overlap) drains the
+// pipeline first: no new packet, no new shift set, and rounds continue until every packet has
+// chased its bulges off the bottom of its block (retire rules below).  The drain plans the lowest
+// packet first; a packet whose window would overlap one already planned is held back a round.  A
+// held packet still hands the scan its chain (its latest window with T = 0, which the chase and
+// update kernels skip), so no deflation is ever made inside one of its bulges.
 template <class Backend>
 int drive(Backend& be, const DriverConfig& cfg, DriverStats& st) {
   const Geom g = geom_for(cfg.p);
   const int n = cfg.n, W = g.W, D = g.D;
-  const long long max_rounds = cfg.max_rounds > 0 ? cfg.max_rounds : 256 + 100LL * n / D;
+  // the reference's budget is maxitfac * n iterations: the round cap scales with maxitfac / 30 and
+  // is 256 + 100 n / D at the default
+  const long long maxitfac = cfg.maxitfac > 0 ? cfg.maxitfac : 30;
+  const long long max_rounds =
+      cfg.max_rounds > 0 ? cfg.max_rounds : std::max(1LL, (256 + 100LL * n / D) * maxitfac / 30);
+  // a packet leaves after at most n / D + 1 rounds; one held back behind a lower packet loses at
+  // most W / D rounds
+  const long long drain_max = (n + W) / D + 4;
   const int lag = std::max(1, cfg.lag);
   const bool trace = be.trace();
   const int max_blocks = std::max(1, std::min(cfg.max_blocks, (int)MS_MAXBLK));
@@ -109,6 +126,13 @@ int drive(Backend& be, const DriverConfig& cfg, DriverStats& st) {
   int next_slot = 0;
   long long pair_counter = 0;     // running index of the next shift pair (taken modulo the set size on the device)
   bool any_set = false;
+  bool draining = false;
+  long long drain_rounds = 0;
+  auto start_drain = [&]() {
+    draining = true;
+    // a packet that has not had its first window yet has not touched the matrix
+    pk.erase(std::remove_if(pk.begin(), pk.end(), [](const Packet& q) { return q.hops == 0; }), pk.end());
+  };
 
   // Shift supply: free running.  A request snapshots the trailing part of a block on the main
   // stream and computes its eigenvalues on a side stream; a packet that is introduced takes the
@@ -195,16 +219,20 @@ int drive(Backend& be, const DriverConfig& cfg, DriverStats& st) {
       }
       pk.resize(k);
     }
-    if (info.done && pk.empty()) {
+    if (!draining && info.done && pk.empty()) {
       // drain the scans still in flight (they cannot undo `done`: zeros are only ever added)
       ScanInfo tmp;
       while (!scan_tickets.empty()) { be.scan_wait(scan_tickets.front(), tmp); scan_tickets.pop_front(); }
       break;
     }
-    if (r > max_rounds) return 1;
+    if (!draining && r > max_rounds) start_drain();
     for (BlockCtl& b : blocks) {
+      if (draining) break;
       const int pass_sets = std::max(1, ((b.ihi - b.ilo + 1) / W) / std::max(1, cfg.nsw / (2 * g.NB)));
-      if (b.idle_sets > 60 + 40 * pass_sets) return 1;
+      if (b.idle_sets > 60 + 40 * pass_sets) {
+        start_drain();
+        break;
+      }
       // ---- shift sets ----
       const int ex_every = 6 + 4 * pass_sets;  // sets without any deflation before the shifts are spread
       double perturb = 0.0;
@@ -233,8 +261,7 @@ int drive(Backend& be, const DriverConfig& cfg, DriverStats& st) {
       }
     }
     // ---- this round's windows ----
-    wins.clear();
-    for (Packet& q : pk) {
+    auto window_of = [&](const Packet& q) {
       WinDesc w;
       w.idle = 0;
       w.ilo = q.ilo; w.ihi = q.ihi; w.nbul = q.nbul; w.pair0 = q.pair0; w.npairs = q.npairs; w.pair_off = q.pair_off;
@@ -249,24 +276,69 @@ int drive(Backend& be, const DriverConfig& cfg, DriverStats& st) {
         const int last_base = w.kbase - 3 * (q.nbul - 1);
         w.T = std::max(1, (q.ihi - 2) - last_base + 1);
       }
-      wins.push_back(w);
+      return w;
+    };
+    wins.clear();
+    std::vector<char> moves(pk.size(), 1);
+    if (!draining) {
+      for (const Packet& q : pk) wins.push_back(window_of(q));
+      // windows of one round must be disjoint (packets of one block keep their distance by
+      // construction; this also covers packets that outlive a split of their block)
+      std::vector<std::pair<int, int>> span;
+      for (const WinDesc& w : wins) span.emplace_back(w.s, w.s + w.wl);
+      std::sort(span.begin(), span.end());
+      for (size_t i = 1; i < span.size() && !draining; i++)
+        if (span[i].first < span[i - 1].second) start_drain();
+    }
+    size_t nmove = pk.size();
+    if (draining) {
+      if (pk.empty()) {
+        ScanInfo tmp;
+        while (!scan_tickets.empty()) { be.scan_wait(scan_tickets.front(), tmp); scan_tickets.pop_front(); }
+        return 1;
+      }
+      if (++drain_rounds > drain_max) return 2;
+      // lowest packet first; one whose window would overlap a window already planned is held back
+      std::vector<size_t> order(pk.size());
+      for (size_t i = 0; i < pk.size(); i++) order[i] = i;
+      std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return pk[a].s > pk[b].s; });
+      wins.clear();
+      moves.assign(pk.size(), 0);
+      std::vector<WinDesc> held;
+      for (size_t i : order) {
+        const WinDesc w = window_of(pk[i]);
+        bool clash = false;
+        for (size_t k = 0; k < pk.size(); k++) {
+          if (!moves[k]) continue;
+          const WinDesc o = window_of(pk[k]);
+          clash |= (w.s < o.s + o.wl && o.s < w.s + w.wl);
+        }
+        if (clash) {
+          WinDesc h = pk[i].last;
+          h.T = 0;  // chain only: the chase and update kernels skip the window, the scan spares the chain
+          held.push_back(h);
+        } else {
+          moves[i] = 1;
+        }
+      }
+      for (size_t i = 0; i < pk.size(); i++)
+        if (moves[i]) wins.push_back(window_of(pk[i]));
+      nmove = wins.size();
+      wins.insert(wins.end(), held.begin(), held.end());
+    }
+    for (size_t i = 0, k = 0; i < pk.size(); i++) {
+      if (!moves[i]) continue;
+      Packet& q = pk[i];
+      q.last = wins[k++];
       q.s = (q.hops == 0) ? q.ilo + D : q.s + D;
       q.hops++;
     }
     if (!wins.empty()) {
-      // windows of one round must be disjoint (packets of one block keep their distance by
-      // construction; this also covers packets that outlive a split of their block)
-      {
-        std::vector<std::pair<int, int>> span;
-        for (const WinDesc& w : wins) span.emplace_back(w.s, w.s + w.wl);
-        std::sort(span.begin(), span.end());
-        for (size_t i = 1; i < span.size(); i++)
-          if (span[i].first < span[i - 1].second) return 1;
-      }
       be.round(wins);
       st.rounds++;
-      st.windows += (long long)wins.size();
-      for (const WinDesc& w : wins) {
+      st.windows += (long long)nmove;
+      for (size_t k = 0; k < nmove; k++) {
+        const WinDesc& w = wins[k];
         const double left = (cfg.wantT ? n : w.ihi + 1) - (w.s + w.wl);
         const double right = w.s - (cfg.wantT ? 0 : w.ilo);
         const double z = cfg.wantZ ? n : 0;

@@ -97,10 +97,13 @@ __global__ void __launch_bounds__(64 * MS_MAXNB, 1) ms_chase_kernel(ChaseParams 
       s_desc.pair_off = slot >= 0 ? slot * 66 : 0;
       s_desc.npairs = slot >= 0 ? ss[MS_SS_NP + slot] : 0;
     }
+    // T = 0: a packet held back by the drain (psd_ms_driver.hpp); only the scan reads the entry
+    if (s_desc.T == 0) s_desc.idle = 1;
     P.wins_dev[blockIdx.x] = s_desc;
   }
   __syncthreads();
   const WinDesc d = s_desc;
+  if (d.T == 0) return;
   const int W = P.g.W, LD = P.g.LD, p = P.p, n = P.n;
   Ctx c;
   c.p = p; c.W = W; c.LD = LD;

@@ -36,17 +36,21 @@ def geom(p):
     return {"W": out[0], "D": out[1], "NB": out[2], "LD": out[3]}
 
 
-def run(H, Z, wantT=True, wantZ=True, nsw=0, rep_max=0):
+def run(H, Z, wantT=True, wantZ=True, nsw=0, rep_max=0, maxitfac=0, max_rounds=0):
     """H, Z: [p][n][n] storage (column-major factors), Hessenberg-triangular / preset Q.
+    maxitfac: the caller's budget factor as psd_rpschur_batched takes it (<= 0: 30);
+    max_rounds > 0: cap on the driver's rounds (the emulated kernels keep working).
     Returns (T, Z, eig, info, stats)."""
     p, n, _ = H.shape
     T = np.ascontiguousarray(H).copy()
     Zo = np.ascontiguousarray(Z).copy() if Z is not None else None
     eig = np.zeros((n, 2))
     info = C.c_int(0)
-    stats = (C.c_longlong * 9)()
+    stats = (C.c_longlong * 10)()
     dp = C.POINTER(C.c_double)
     lib().ms_emul_run(n, p, T.ctypes.data_as(dp), Zo.ctypes.data_as(dp) if Zo is not None else None,
-                      int(wantT), int(wantZ), nsw, rep_max, eig.ctypes.data_as(dp), C.byref(info), stats)
-    names = ["sweeps", "rounds", "windows", "shift_pairs", "exceptional", "final_blocks", "bulge_steps", "status", "bulges_left_behind"]
+                      int(wantT), int(wantZ), nsw, rep_max, int(maxitfac), C.c_longlong(max_rounds),
+                      eig.ctypes.data_as(dp), C.byref(info), stats)
+    names = ["sweeps", "rounds", "windows", "shift_pairs", "exceptional", "final_blocks", "bulge_steps", "status",
+             "bulges_left_behind", "held_windows"]
     return T, Zo, eig[:, 0] + 1j * eig[:, 1], info.value, dict(zip(names, list(stats)))

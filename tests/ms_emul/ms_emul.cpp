@@ -175,7 +175,7 @@ struct EmuBackend {
     }
   }
 
-  long long max_rounds = -1, nrounds = 0;
+  long long max_rounds = -1, nrounds = 0, held_windows = 0;
   bool skip_apply = false;
   void round(const std::vector<WinDesc>& wins_) {
     if (max_rounds >= 0 && nrounds >= max_rounds) return;
@@ -186,6 +186,10 @@ struct EmuBackend {
     std::vector<double> Hw((size_t)p * W * LD), Uw((size_t)p * W * LD);
     for (int w = 0; w < cnt; w++) {
       WinDesc& dd = plan[off + w];
+      if (dd.T == 0) {  // packet held back: the CUDA chase kernel returns at once
+        held_windows++;
+        continue;
+      }
       if (dd.intro) {  // newest complete shift set of this block, as the CUDA kernel picks it
         int best = -1, bseq = 0, any = -1, aseq = 0;
         for (int k = 0; k < 8; k++) {
@@ -264,7 +268,10 @@ struct EmuBackend {
           }
       }
     }
-    apply(plan.data() + off, cnt);
+    std::vector<WinDesc> moved;  // (held-back packets have no update)
+    for (const WinDesc& d : plan)
+      if (d.T != 0) moved.push_back(d);
+    apply(moved.data(), (int)moved.size());
   }
 
   double junk = 0.0;  // largest entry below the Hessenberg / triangular structure when the pipeline ends
@@ -333,12 +340,16 @@ struct EmuBackend {
 extern "C" {
 
 // H: [p][n*n] column-major Hessenberg-triangular factors (rightwards order), Z: [p][n*n] preset
-// Schur vectors or NULL.  stats[9] (last: 1 if a bulge was left behind when the pipeline ended): sweeps, rounds, windows, shift pairs, exceptional, final
-// blocks, bulge steps, status.  Returns the status of the driver (0 = finished).
+// Schur vectors or NULL.  maxitfac: the caller's budget factor (<= 0: 30).  max_rounds > 0 caps the
+// driver's rounds (DriverConfig::max_rounds; the backend keeps working, so a give-up drains).
+// stats[10]: sweeps, rounds, windows, shift pairs, exceptional, final blocks, bulge steps, status,
+// 1 if a bulge was left behind when the pipeline finished, windows held back by the drain.
+// Returns the status of the driver (0 = finished).
 int ms_emul_run(int n, int p, double* Hbuf, double* Zbuf, int wantT, int wantZ, int nsw, int rep_max,
-                double* eig, int* info, long long* stats) {
+                int maxitfac, long long max_rounds, double* eig, int* info, long long* stats) {
   EmuBackend be;
-  be.n = n; be.p = p; be.wantT = wantT; be.wantZ = (wantZ && Zbuf) ? 1 : 0; be.maxitfac = 30;
+  be.n = n; be.p = p; be.wantT = wantT; be.wantZ = (wantZ && Zbuf) ? 1 : 0;
+  be.maxitfac = maxitfac > 0 ? maxitfac : 30;
   be.g = geom_for(p);
   for (int j = 0; j < p; j++) {
     be.H.push_back(Hbuf + (size_t)j * n * n);
@@ -350,6 +361,8 @@ int ms_emul_run(int n, int p, double* Hbuf, double* Zbuf, int wantT, int wantZ, 
   cfg.n = n; cfg.p = p; cfg.wantT = wantT; cfg.wantZ = be.wantZ;
   if (nsw > 0) cfg.nsw = nsw;
   if (rep_max > 0) cfg.rep_max = rep_max;
+  cfg.maxitfac = maxitfac;
+  if (max_rounds > 0) cfg.max_rounds = max_rounds;
   if (const char* ev = getenv("MS_EMUL_MAXROUNDS")) {
     be.max_rounds = atoll(ev);
     cfg.max_rounds = be.max_rounds + 4;
@@ -360,11 +373,12 @@ int ms_emul_run(int n, int p, double* Hbuf, double* Zbuf, int wantT, int wantZ, 
   if (const char* ev = getenv("MS_EMUL_AHEAD")) cfg.sets_ahead = atoi(ev);
   DriverStats ds;
   const int status = drive(be, cfg, ds);
-  *info = be.info;
+  *info = (status == 2) ? n : be.info;  // as psd_ms.cu reports a drain that did not end
   if (stats) {
     stats[0] = ds.sweeps; stats[1] = ds.rounds; stats[2] = ds.windows; stats[3] = ds.shift_pairs;
     stats[4] = ds.exceptional; stats[5] = ds.final_blocks; stats[6] = be.chase_steps; stats[7] = status;
     stats[8] = (be.junk != 0.0) ? 1 : 0;
+    stats[9] = be.held_windows;
   }
   return status;
 }
