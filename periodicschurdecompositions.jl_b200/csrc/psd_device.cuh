@@ -22,12 +22,17 @@ namespace psd {
 
 #define PSD_DEV __device__ __forceinline__
 
-// exact power-of-two scale s = 2^-ilogb(m) for m > 0 (handles denormals)
-PSD_DEV double pow2_rescale(double m) {
+// exponent s of the exact power-of-two scale 2^s that brings m > 0 into [0.5, 1), capped at 1000
+// because 2^-e itself overflows for subnormal m.  A caller that records the scale of a factor must
+// record this s, not -e: below 2^-1000 the two differ.
+PSD_DEV int pow2_shift(double m) {
   int e;
   (void)frexp(m, &e);  // m = f * 2^e, f in [0.5,1)
-  return scalbn(1.0, (-e > 1000) ? 1000 : -e);  // 2^-e itself overflows for subnormal m
+  return (-e > 1000) ? 1000 : -e;
 }
+
+// exact power-of-two scale s = 2^-ilogb(m) for m > 0 (handles denormals)
+PSD_DEV double pow2_rescale(double m) { return scalbn(1.0, pow2_shift(m)); }
 
 // Reflector for a 2- or 3-vector held in registers.  On return x0 = beta, (v1,v2) the
 // essential part, tau returned.  Same mathematics as householder.jl:66-108 (dlarfg); the

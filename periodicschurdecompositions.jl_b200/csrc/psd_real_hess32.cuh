@@ -192,14 +192,13 @@ __global__ void __launch_bounds__(256) rphess_warp32_kernel_t(Hess32Params P) {
       if (lane < n)
         for (int c = 0; c < n; c++) m = fmax(m, fabs(dst[c * ld + lane]));
       m = warp_max(m);
-      if (m > 0.0 && m < 1.7e308) {
-        int e;
-        (void)frexp(m, &e);
-        if (e != 0) {
-          const double sc = scalbn(1.0, (-e > 1000) ? 1000 : -e);
+      if (m > 0.0 && m <= DBL_MAX) {
+        const int s = pow2_shift(m);
+        if (s != 0) {
+          const double sc = scalbn(1.0, s);
           if (lane < n)
             for (int c = 0; c < n; c++) dst[c * ld + lane] *= sc;
-          escale += e;
+          escale -= s;
         }
       }
     }
@@ -362,14 +361,13 @@ __global__ void __launch_bounds__(512) rphess_pair32_kernel_t(Hess32Params P) {
       if (lane < n)
         for (int c = 0; c < n; c++) m = fmax(m, fabs(dst[c * ld + lane]));
       m = warp_max(m);
-      if (m > 0.0 && m < 1.7e308) {
-        int e;
-        (void)frexp(m, &e);
-        if (e != 0) {
-          const double sc = scalbn(1.0, (-e > 1000) ? 1000 : -e);
+      if (m > 0.0 && m <= DBL_MAX) {
+        const int s = pow2_shift(m);
+        if (s != 0) {
+          const double sc = scalbn(1.0, s);
           if (lane < n)
             for (int c = 0; c < n; c++) dst[c * ld + lane] *= sc;
-          escale += e;
+          escale -= s;
         }
       }
     }
@@ -692,14 +690,13 @@ __global__ void __launch_bounds__(AHEAD_WARPS * 32 * 4) rphess_ahead32_kernel_t(
       if (lane < n)
         for (int c = 0; c < n; c++) m = fmax(m, fabs(dst[c * ld + lane]));
       m = warp_max(m);
-      if (m > 0.0 && m < 1.7e308) {
-        int e;
-        (void)frexp(m, &e);
-        if (e != 0) {
-          const double sc = scalbn(1.0, (-e > 1000) ? 1000 : -e);
+      if (m > 0.0 && m <= DBL_MAX) {
+        const int s = pow2_shift(m);
+        if (s != 0) {
+          const double sc = scalbn(1.0, s);
           if (lane < n)
             for (int c = 0; c < n; c++) dst[c * ld + lane] *= sc;
-          escale += e;
+          escale -= s;
         }
       }
     }

@@ -295,11 +295,10 @@ __global__ void rpschur_kernel(RpschurParams P) {
         const double* src = c.Hp(j);
         const double m = c.hnorms[j];
         double sc = 1.0;
-        if (m > 0.0 && m < 1.7e308) {
-          int e;
-          (void)frexp(m, &e);
-          sc = scalbn(1.0, (-e > 1000) ? 1000 : -e);
-          escale += e;
+        if (m > 0.0 && m <= DBL_MAX) {
+          const int s = pow2_shift(m);
+          sc = scalbn(1.0, s);
+          escale -= s;
         }
         for (int e = tid; e < (int)nn; e += nt) {
           int r = e % n, cc = e / n;
