@@ -11,6 +11,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
+#include <initializer_list>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -56,19 +58,20 @@ int fail(int code, const std::string& msg) {
 
 constexpr int kSlotsPerDevice = 3;
 
+// Roles of the pipeline buffers of a batched host call: the factors (A in, T out), Z, the
+// eigenvalues (real: eig in kVal0; generalized: alpha, beta, alphascale), info, iteration counts.
+enum Role { kFactors, kZ, kVal0, kVal1, kVal2, kInfo, kIters, kRoles };
+
 struct Slot {
   cudaStream_t stream = nullptr;
-  double* dA = nullptr;
-  double* dZ = nullptr;
-  double* dEig = nullptr;
-  int32_t* dInfo = nullptr;
-  size_t capA = 0, capZ = 0, capEig = 0, capInfo = 0;
-  // pinned staging (only used when the caller's buffers are pageable)
-  double* hA = nullptr;
-  double* hZ = nullptr;
-  double* hEig = nullptr;
-  int32_t* hInfo = nullptr;
-  size_t hcapA = 0, hcapZ = 0, hcapEig = 0, hcapInfo = 0;
+  // pipeline buffers by role: device, and pinned staging (only used when the caller's buffers are
+  // pageable); the pipeline copies these out, so no launch function uses them as scratch
+  void* dBuf[kRoles] = {};
+  size_t dCap[kRoles] = {};
+  void* hBuf[kRoles] = {};
+  size_t hCap[kRoles] = {};
+  double* dArg[3] = {};  // operands of the single-slot entry points (rphess_packed, rowwise, dgemm)
+  size_t capArg[3] = {};
   unsigned long long* dCounter = nullptr;  // [2]: reduction kernel, QR kernel
   double* dScratch = nullptr;
   size_t capScratch = 0;
@@ -77,19 +80,13 @@ struct Slot {
   double* dPk[8] = {nullptr};  // packed leading parts handed to the later occupancy phases
   size_t capPk[8] = {0};
   unsigned long long* dPhaseCtr = nullptr;  // work counters of the phase launches
-  // generalized paths: alpha, beta, alphascale (device + pinned staging) and the signature
-  void* dX[3] = {nullptr, nullptr, nullptr};
-  size_t capX[3] = {0, 0, 0};
-  void* hX[3] = {nullptr, nullptr, nullptr};
-  size_t hcapX[3] = {0, 0, 0};
-  unsigned char* dS = nullptr;
+  unsigned char* dS = nullptr;  // generalized paths: the signature
   size_t capS = 0;
   psd::ms::Workspace* ms = nullptr;  // large-N multishift iteration (psd_ms.cu)
-  // iteration counts (psd_set_iters_output): device buffer, pinned staging, and the pointer the
-  // launch functions read for the chunk being enqueued (nullptr: not wanted)
-  int32_t* dIters = nullptr;
-  int32_t* hIters = nullptr;
-  size_t capIters = 0, hcapIters = 0;
+  void* dTeam[3] = {};  // team iteration scratch: alpha, beta, alphascale
+  size_t capTeam[3] = {};
+  // iteration counts (psd_set_iters_output) of the chunk being enqueued, read by the launch
+  // functions (nullptr: not wanted)
   int32_t* curIters = nullptr;
   double* curTau = nullptr;  // psd_rphess_packed_batched: device tau of the chunk being enqueued
   long long* dProf = nullptr;        // PSD_PANEL_PROF cycle counters (debug builds)
@@ -156,6 +153,17 @@ bool is_pinned(const void* p) {
     return false;
   }
   return at.type == cudaMemoryTypeHost || at.type == cudaMemoryTypeManaged;
+}
+
+// The single-slot entry points run on slot 0 of the handle's first device: make that device
+// current and wait until the slot's stream is idle.
+int use_slot0(psd_handle_s* h) {
+  Device& dev = h->devs[0];
+  PSD_CUDA(cudaSetDevice(dev.ordinal));
+  Slot& s = dev.slots[0];
+  if (!s.stream) PSD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
+  PSD_CUDA(cudaStreamSynchronize(s.stream));
+  return PSD_OK;
 }
 
 // Bracket a kernel launch with CUDA events on its stream when profiling is enabled.
@@ -534,16 +542,16 @@ int launch_team_iteration(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t 
   const bool wantZ = rc.wantZ && dZ;
   int e;
   const size_t cnt = (size_t)batch * n;
-  if ((e = ensure_dev(aux.dX[0], aux.capX[0], cnt * 16))) return e;
-  if ((e = ensure_dev(aux.dX[1], aux.capX[1], cnt * 8))) return e;
-  if ((e = ensure_dev(aux.dX[2], aux.capX[2], cnt * 8))) return e;
+  if ((e = ensure_dev(aux.dTeam[0], aux.capTeam[0], cnt * 16))) return e;
+  if ((e = ensure_dev(aux.dTeam[1], aux.capTeam[1], cnt * 8))) return e;
+  if ((e = ensure_dev(aux.dTeam[2], aux.capTeam[2], cnt * 8))) return e;
   psd::GpqzParams<double> P;
   P.n = n; P.p = p; P.batch = batch; P.left = rc.left; P.wantT = rc.wantT; P.wantZ = wantZ ? 1 : 0;
   P.maxitfac = 4 * (rc.maxitfac > 0 ? rc.maxitfac : 30);  // QZ loop counts deflation steps too (rgeneralized.jl:52)
   P.skip_reduce = 1; P.reduce_only = 0;
   P.S = nullptr;
   P.A = dA; P.Z = wantZ ? dZ : nullptr;
-  P.alpha = (psd::cplx*)aux.dX[0]; P.beta = (double*)aux.dX[1]; P.scale = (long long*)aux.dX[2];
+  P.alpha = (psd::cplx*)aux.dTeam[0]; P.beta = (double*)aux.dTeam[1]; P.scale = (long long*)aux.dTeam[2];
   P.info = dInfo;
   P.use_smem = 0; P.ldh = n; P.debug = 0; P.counter = nullptr; P.blocked_stage1 = 0; P.windowed_stage2 = 0; P.windowed_qz = 0;
   P.deep = 4;  // team mode: < 1 element pair per thread and factor, one pass instead of p + 1 (N = 1024: 7.1 s -> 5.3 s)
@@ -567,7 +575,7 @@ int launch_team_iteration(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t 
     PSD_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(ctas), dim3(256), args, smem, stream));
   }
   psd::gvalues_kernel<<<std::min<long long>(1024, (long long)(cnt + 255) / 256), 256, 0, stream>>>(
-      (const psd::cplx*)aux.dX[0], (const double*)aux.dX[1], (const long long*)aux.dX[2], dEig, (long long)cnt);
+      (const psd::cplx*)aux.dTeam[0], (const double*)aux.dTeam[1], (const long long*)aux.dTeam[2], dEig, (long long)cnt);
   PSD_CUDA(cudaGetLastError());
   __atomic_fetch_add(&h->stats[0], (int64_t)2, __ATOMIC_RELAXED);
   return PSD_OK;
@@ -694,161 +702,115 @@ int drain_slots(Device& dev, int code) {
       return drain_slots(dev, fail(PSD_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e__))); \
   } while (0)
 
-// One device's share of a host-buffer batched call.
-int run_real_shard(psd_handle_s* h, Device& dev, const RealCall& rc, long long first, long long count,
-                   double* A, double* Z, double* eig, int32_t* info, bool pinned,
-                   int64_t* bytes_h2d, int64_t* bytes_d2h) {
-  if (count <= 0) return PSD_OK;
-  PSD_SHARD_CUDA(cudaSetDevice(dev.ordinal));
-  const size_t nn = (size_t)rc.n * rc.n;
-  const size_t per = nn * rc.p;  // doubles per problem
-  const bool wantZ = rc.wantZ && Z;
-  const bool outT = rc.wantT || rc.reduce_only;
-  // Chunks grow geometrically (x4) from 1/16 of the full size up to ~2 GiB of factors: the first
-  // host-to-device copy is the only one no kernel overlaps, so it is kept short, while the large
-  // later chunks amortise the tail of the persistent kernels (measured on config 2).
-  long long chunk = std::max<long long>(1, (2048LL << 20) / (long long)(per * sizeof(double)));
-  if (!pinned) chunk = std::max<long long>(1, std::min<long long>(chunk, (512LL << 20) / (long long)(per * sizeof(double))));
-  chunk = std::min(chunk, count);
-  // pageable buffers are staged through pinned ones by the host: at least four chunks, so that the
-  // host copies of one chunk overlap the device work of the others
-  if (!pinned && (size_t)count * per * sizeof(double) >= (64u << 20) && count >= 8)
-    chunk = std::min(chunk, (count + 3) / 4);
-  int si = 0;
-  int rcode = PSD_OK;
-  // results of a pageable call that still sit in a slot's pinned buffers
+// One host array of a batched call as the pipeline copies it: problem b's part starts at
+// host + b * per.
+struct HostArray {
+  char* host;           // nullptr: a device buffer the kernels write but the call does not return
+  size_t per;           // bytes per problem
+  Role role;            // the slot buffers it goes through
+  bool pinned = true;   // false: staged even when the call runs pinned
+  bool counted = true;  // counted in the h2d / d2h bytes
+};
+
+// Enqueues the kernels of one chunk of nb problems on the slot's stream; d[role] is the chunk's
+// device buffer of each listed array (nullptr for the other roles).
+using LaunchFn = std::function<int(Slot& s, long long nb, void* const* d)>;
+
+// One device's share of a batched host call: the problems from `first` on, in `chunks`.  Chunk c
+// runs on slot c % kSlotsPerDevice.  A pinned call copies the caller's buffers in place; otherwise
+// they go through the slot's pinned staging buffers.  `in` lists the factors first.
+int run_shard(Device& dev, long long first, const std::vector<long long>& chunks, bool pinned,
+              const std::vector<HostArray>& in, const std::vector<HostArray>& out, const LaunchFn& launch,
+              int64_t* bytes_h2d, int64_t* bytes_d2h) {
+  // chunks above this size are copied straight from / to pageable memory (no pinned staging copy)
+  const size_t kStageLimit = 1ULL << 30;
+  // results of a staged chunk that still sit in a slot's pinned buffers: copied out when the slot
+  // is drained (before its next use, or at the end), so that the host copies overlap the device
+  // work of the other slots
   struct Pending {
-    bool any = false;
-    double *dstA = nullptr, *dstZ = nullptr, *dstEig = nullptr;
-    int32_t *dstInfo = nullptr, *dstIters = nullptr;
-    size_t bytesA = 0, bytesEig = 0, bytesInfo = 0, bytesIters = 0;
-  } pend[kSlotsPerDevice];
-  auto flush = [&](int k) {
-    Pending& q = pend[k];
-    if (!q.any) return;
-    Slot& s = dev.slots[k];
-    if (q.dstA) std::memcpy(q.dstA, s.hA, q.bytesA);
-    if (q.dstZ) std::memcpy(q.dstZ, s.hZ, q.bytesA);
-    if (q.dstEig) std::memcpy(q.dstEig, s.hEig, q.bytesEig);
-    if (q.dstInfo) std::memcpy(q.dstInfo, s.hInfo, q.bytesInfo);
-    if (q.dstIters) std::memcpy(q.dstIters, s.hIters, q.bytesIters);
-    q = Pending();
+    char* dst;
+    const void* src;
+    size_t bytes;
   };
-  long long nb = 0, next = (count > chunk) ? std::max<long long>(1, chunk / (pinned ? 16 : 2)) : chunk;
-  for (long long off = 0; off < count && rcode == PSD_OK; off += nb, si = (si + 1) % kSlotsPerDevice) {
-    nb = std::min(next, count - off);
-    next = std::min(chunk, next * 4);
+  std::vector<Pending> pend[kSlotsPerDevice];
+  auto flush = [&](int k) {
+    for (const Pending& q : pend[k]) std::memcpy(q.dst, q.src, q.bytes);
+    pend[k].clear();
+  };
+  long long off = first;
+  for (size_t c = 0; c < chunks.size(); off += chunks[c++]) {
+    const long long nb = chunks[c];
+    const int si = (int)(c % kSlotsPerDevice);
     Slot& s = dev.slots[si];
     if (!s.stream) PSD_SHARD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
     // the slot's previous chunk must have fully drained before its buffers are reused
     PSD_SHARD_CUDA(cudaStreamSynchronize(s.stream));
     flush(si);
+    const bool big = nb * in[0].per > kStageLimit;
+    auto staged = [&](const HostArray& a) { return pinned ? !a.pinned : !big; };
     int e;
-    if ((e = ensure_dev(s.dA, s.capA, nb * per * sizeof(double)))) return drain_slots(dev, e);
-    if (wantZ && (e = ensure_dev(s.dZ, s.capZ, nb * per * sizeof(double)))) return drain_slots(dev, e);
-    if ((e = ensure_dev(s.dEig, s.capEig, nb * 2 * rc.n * sizeof(double)))) return drain_slots(dev, e);
-    if ((e = ensure_dev(s.dInfo, s.capInfo, nb * sizeof(int32_t)))) return drain_slots(dev, e);
-    double* srcA = A + (size_t)(first + off) * per;
-    const size_t bytesA = nb * per * sizeof(double);
-    if (pinned) {
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.dA, srcA, bytesA, cudaMemcpyHostToDevice, s.stream));
-    } else {
-      if ((e = ensure_pinned(s.hA, s.hcapA, bytesA))) return drain_slots(dev, e);
-      std::memcpy(s.hA, srcA, bytesA);
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.dA, s.hA, bytesA, cudaMemcpyHostToDevice, s.stream));
-    }
-    *bytes_h2d += (int64_t)bytesA;
-    const bool wantIters = h->iters_host && !rc.reduce_only;
-    const size_t bytesIters = nb * sizeof(int32_t);
-    s.curIters = nullptr;
-    if (wantIters) {
-      if ((e = ensure_dev(s.dIters, s.capIters, bytesIters))) return drain_slots(dev, e);
-      if ((e = ensure_pinned(s.hIters, s.hcapIters, bytesIters))) return drain_slots(dev, e);
-      PSD_SHARD_CUDA(cudaMemsetAsync(s.dIters, 0, bytesIters, s.stream));
-      s.curIters = s.dIters;
-    }
-    if (wantZ && rc.z_preset) {
-      // Z enters as the caller's Q_j (accumulated onto)
-      double* srcZ = Z + (size_t)(first + off) * per;
-      if (pinned) {
-        PSD_SHARD_CUDA(cudaMemcpyAsync(s.dZ, srcZ, bytesA, cudaMemcpyHostToDevice, s.stream));
-      } else {
-        if ((e = ensure_pinned(s.hZ, s.hcapZ, bytesA))) return drain_slots(dev, e);
-        std::memcpy(s.hZ, srcZ, bytesA);
-        PSD_SHARD_CUDA(cudaMemcpyAsync(s.dZ, s.hZ, bytesA, cudaMemcpyHostToDevice, s.stream));
+    void* d[kRoles] = {};
+    for (const auto* list : {&in, &out})
+      for (const HostArray& a : *list) {
+        if ((e = ensure_dev(s.dBuf[a.role], s.dCap[a.role], nb * a.per))) return drain_slots(dev, e);
+        d[a.role] = s.dBuf[a.role];
       }
-      *bytes_h2d += (int64_t)bytesA;
+    for (const HostArray& a : in) {
+      const char* src = a.host + off * a.per;
+      const size_t bytes = nb * a.per;
+      const bool st = staged(a);
+      if (st) {
+        if ((e = ensure_pinned(s.hBuf[a.role], s.hCap[a.role], bytes))) return drain_slots(dev, e);
+        std::memcpy(s.hBuf[a.role], src, bytes);
+      }
+      PSD_SHARD_CUDA(cudaMemcpyAsync(d[a.role], st ? s.hBuf[a.role] : src, bytes, cudaMemcpyHostToDevice, s.stream));
+      if (a.counted) *bytes_h2d += (int64_t)bytes;
     }
-    e = launch_real(h, dev, s, s.stream, rc, nb, s.dA, wantZ ? s.dZ : nullptr, s.dEig, s.dInfo);
-    s.curIters = nullptr;
-    if (e) return drain_slots(dev, e);
-    if (wantIters) {
-      // always through the slot's pinned buffer; copied out when the slot is drained
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.hIters, s.dIters, bytesIters, cudaMemcpyDeviceToHost, s.stream));
-      pend[si].any = true;
-      pend[si].dstIters = h->iters_host + (first + off);
-      pend[si].bytesIters = bytesIters;
+    if ((e = launch(s, nb, d))) return drain_slots(dev, e);
+    for (const HostArray& a : out) {
+      if (!a.host) continue;
+      char* dst = a.host + off * a.per;
+      const size_t bytes = nb * a.per;
+      const bool st = staged(a);
+      if (st && (e = ensure_pinned(s.hBuf[a.role], s.hCap[a.role], bytes))) return drain_slots(dev, e);
+      PSD_SHARD_CUDA(cudaMemcpyAsync(st ? s.hBuf[a.role] : dst, d[a.role], bytes, cudaMemcpyDeviceToHost, s.stream));
+      if (st) pend[si].push_back({dst, s.hBuf[a.role], bytes});
+      if (a.counted) *bytes_d2h += (int64_t)bytes;
     }
-    // results
-    double* dstEig = eig ? eig + (size_t)(first + off) * 2 * rc.n : nullptr;
-    int32_t* dstInfo = info ? info + (first + off) : nullptr;
-    double* dstZ = wantZ ? Z + (size_t)(first + off) * per : nullptr;
-    const size_t bytesEig = nb * 2 * rc.n * sizeof(double);
-    const size_t bytesInfo = nb * sizeof(int32_t);
-    if (pinned) {
-      if (outT) PSD_SHARD_CUDA(cudaMemcpyAsync(srcA, s.dA, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      if (wantZ) PSD_SHARD_CUDA(cudaMemcpyAsync(dstZ, s.dZ, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      if (dstEig) PSD_SHARD_CUDA(cudaMemcpyAsync(dstEig, s.dEig, bytesEig, cudaMemcpyDeviceToHost, s.stream));
-      if (dstInfo) PSD_SHARD_CUDA(cudaMemcpyAsync(dstInfo, s.dInfo, bytesInfo, cudaMemcpyDeviceToHost, s.stream));
-    } else {
-      if (wantZ && (e = ensure_pinned(s.hZ, s.hcapZ, bytesA))) return drain_slots(dev, e);
-      if ((e = ensure_pinned(s.hEig, s.hcapEig, bytesEig))) return drain_slots(dev, e);
-      if ((e = ensure_pinned(s.hInfo, s.hcapInfo, bytesInfo))) return drain_slots(dev, e);
-      if (outT) PSD_SHARD_CUDA(cudaMemcpyAsync(s.hA, s.dA, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      if (wantZ) PSD_SHARD_CUDA(cudaMemcpyAsync(s.hZ, s.dZ, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.hEig, s.dEig, bytesEig, cudaMemcpyDeviceToHost, s.stream));
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.hInfo, s.dInfo, bytesInfo, cudaMemcpyDeviceToHost, s.stream));
-      // pageable destination: copied out of the pinned buffers when the slot is drained (before its
-      // next use, or at the end), so that the host copies overlap the device work of the other slots
-      Pending& q = pend[si];  // (dstIters may already be set)
-      q.any = true;
-      q.dstA = outT ? srcA : nullptr;
-      q.dstZ = wantZ ? dstZ : nullptr;
-      q.dstEig = dstEig;
-      q.dstInfo = dstInfo;
-      q.bytesA = bytesA; q.bytesEig = bytesEig; q.bytesInfo = bytesInfo;
-    }
-    *bytes_d2h += (int64_t)((outT ? bytesA : 0) + (wantZ ? bytesA : 0) + bytesEig + bytesInfo);
   }
   for (int k = 0; k < kSlotsPerDevice; k++)
     if (dev.slots[k].stream) {
       PSD_SHARD_CUDA(cudaStreamSynchronize(dev.slots[k].stream));
       flush(k);
     }
-  return rcode;
+  return PSD_OK;
 }
 
-int run_real_host(psd_handle_t h, const RealCall& rc, int64_t batch, double* A, double* Z, double* eig,
-                  int32_t* info) {
-  if (!h) return fail(PSD_ERR_BAD_ARG, "null handle");
-  if (rc.n < 1 || rc.p < 1 || batch < 0) return fail(PSD_ERR_BAD_ARG, "n, p must be >= 1 and batch >= 0");
-  if (!A) return fail(PSD_ERR_BAD_ARG, "A must not be NULL");
-  if (!rc.reduce_only && (!eig || !info)) return fail(PSD_ERR_BAD_ARG, "eig and info must not be NULL");
-  if (rc.wantZ && !Z) return fail(PSD_ERR_BAD_ARG, "wantZ set but Z is NULL");
-  if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
+// Runs one device's share [first, first + count) of a batched host call, on the current device.
+using ShardFn = std::function<int(Device& dev, long long first, long long count, bool pinned, int64_t* bytes_h2d,
+                                  int64_t* bytes_d2h)>;
+
+// A batched host call: one contiguous range of the batch per device of the handle, each on a host
+// thread of its own.  The call runs pinned when every buffer in `args` is page-locked.
+int run_host(psd_handle_s* h, int64_t batch, std::initializer_list<const void*> args, const ShardFn& shard) {
   std::lock_guard<std::mutex> lock(h->mu);
   for (auto& s : h->stats) s = 0;
   if (batch == 0) return PSD_OK;
-  const bool pinned = is_pinned(A) && is_pinned(Z) && is_pinned(eig) && is_pinned(info);
+  bool pinned = true;
+  for (const void* a : args) pinned = pinned && is_pinned(a);
   const int nd = (int)h->devs.size();
   std::vector<int> codes(nd, PSD_OK);
   std::vector<std::string> msgs(nd);
   std::vector<int64_t> h2d(nd, 0), d2h(nd, 0);
   auto t0 = std::chrono::steady_clock::now();
-  auto work = [&](int d) {
+  auto run_device = [&](int d) -> int {
     const long long lo = batch * d / nd, hi = batch * (d + 1) / nd;
-    codes[d] = run_real_shard(h, h->devs[d], rc, lo, hi - lo, A, Z, eig, info, pinned, &h2d[d], &d2h[d]);
-    if (codes[d]) msgs[d] = g_err;
+    if (hi == lo) return PSD_OK;
+    PSD_CUDA(cudaSetDevice(h->devs[d].ordinal));
+    return shard(h->devs[d], lo, hi - lo, pinned, &h2d[d], &d2h[d]);
+  };
+  auto work = [&](int d) {
+    if ((codes[d] = run_device(d))) msgs[d] = g_err;
   };
   if (nd == 1) {
     work(0);
@@ -868,10 +830,69 @@ int run_real_host(psd_handle_t h, const RealCall& rc, int64_t batch, double* A, 
   return PSD_OK;
 }
 
+// Chunk sizes of the real standard path for `count` problems of `per` bytes of factors.
+// Chunks grow geometrically (x4) from 1/16 of the full size up to ~2 GiB of factors: the first
+// host-to-device copy is the only one no kernel overlaps, so it is kept short, while the large
+// later chunks amortise the tail of the persistent kernels (measured on config 2).
+std::vector<long long> plan_real_chunks(long long count, size_t per, bool pinned) {
+  long long chunk = std::max<long long>(1, (2048LL << 20) / (long long)per);
+  if (!pinned) chunk = std::max<long long>(1, std::min<long long>(chunk, (512LL << 20) / (long long)per));
+  chunk = std::min(chunk, count);
+  // pageable buffers are staged through pinned ones by the host: at least four chunks, so that the
+  // host copies of one chunk overlap the device work of the others
+  if (!pinned && (size_t)count * per >= (64u << 20) && count >= 8)
+    chunk = std::min(chunk, (count + 3) / 4);
+  std::vector<long long> chunks;
+  long long next = (count > chunk) ? std::max<long long>(1, chunk / (pinned ? 16 : 2)) : chunk;
+  for (long long off = 0; off < count; off += chunks.back()) {
+    chunks.push_back(std::min(next, count - off));
+    next = std::min(chunk, next * 4);
+  }
+  return chunks;
+}
+
+int run_real_host(psd_handle_t h, const RealCall& rc, int64_t batch, double* A, double* Z, double* eig,
+                  int32_t* info) {
+  if (!h) return fail(PSD_ERR_BAD_ARG, "null handle");
+  if (rc.n < 1 || rc.p < 1 || batch < 0) return fail(PSD_ERR_BAD_ARG, "n, p must be >= 1 and batch >= 0");
+  if (!A) return fail(PSD_ERR_BAD_ARG, "A must not be NULL");
+  if (!rc.reduce_only && (!eig || !info)) return fail(PSD_ERR_BAD_ARG, "eig and info must not be NULL");
+  if (rc.wantZ && !Z) return fail(PSD_ERR_BAD_ARG, "wantZ set but Z is NULL");
+  if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
+  const size_t per = (size_t)rc.n * rc.n * rc.p * sizeof(double);  // bytes of factors per problem
+  const bool wantZ = rc.wantZ && Z;
+  return run_host(h, batch, {A, Z, eig, info}, [&](Device& dev, long long first, long long count, bool pinned,
+                                                   int64_t* bytes_h2d, int64_t* bytes_d2h) {
+    std::vector<HostArray> in{{(char*)A, per, kFactors}}, out;
+    if (wantZ && rc.z_preset) in.push_back({(char*)Z, per, kZ});  // Z enters as the caller's Q_j (accumulated onto)
+    if (rc.wantT || rc.reduce_only) out.push_back({(char*)A, per, kFactors});
+    if (wantZ) out.push_back({(char*)Z, per, kZ});
+    if (!rc.reduce_only) {
+      out.push_back({(char*)eig, 2 * rc.n * sizeof(double), kVal0});
+      out.push_back({(char*)info, sizeof(int32_t), kInfo});
+      // the iteration counts are a setting of the handle, not an argument of the call: they do not
+      // decide whether the call runs pinned, and the byte counters leave them out
+      int32_t* it = h->iters_host;
+      if (it) out.push_back({(char*)it, sizeof(int32_t), kIters, is_pinned(it), false});
+    }
+    auto launch = [&](Slot& s, long long nb, void* const* d) -> int {
+      int32_t* iters = (int32_t*)d[kIters];
+      if (iters) PSD_CUDA(cudaMemsetAsync(iters, 0, nb * sizeof(int32_t), s.stream));
+      s.curIters = iters;
+      const int e = launch_real(h, dev, s, s.stream, rc, nb, (double*)d[kFactors], (double*)d[kZ],
+                                (double*)d[kVal0], (int32_t*)d[kInfo]);
+      s.curIters = nullptr;
+      return e;
+    };
+    return run_shard(dev, first, plan_real_chunks(count, per, pinned), pinned, in, out, launch, bytes_h2d,
+                     bytes_d2h);
+  });
+}
+
 
 // ---------------------------------------------------------------------------------------------
-// Generalized paths (complex periodic QZ; real periodic QZ): same sharding / chunking / slot
-// pipeline as the real standard path, with (alpha, beta, alphascale) instead of eig.
+// Generalized paths (complex periodic QZ; real periodic QZ): the pipeline of the real standard
+// path with a chunk policy of their own, and (alpha, beta, alphascale) instead of eig.
 // ---------------------------------------------------------------------------------------------
 struct GenCall {
   int n, p, left, wantT, wantZ, maxitfac, skip_reduce;
@@ -976,115 +997,20 @@ int launch_gen(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t stream, con
   return launch_gen_t<double>(h, dev, aux, stream, gc, batch, dA, dZ, dAlpha, dBeta, dScale, dInfo);
 }
 
-int run_gen_shard(psd_handle_s* h, Device& dev, const GenCall& gc, long long first, long long count, char* A,
-                  char* Z, char* alpha, char* beta, int64_t* scale, int32_t* info, bool pinned,
-                  int64_t* bytes_h2d, int64_t* bytes_d2h) {
-  if (count <= 0) return PSD_OK;
-  PSD_SHARD_CUDA(cudaSetDevice(dev.ordinal));
-  const size_t es = gen_elem(gc);
-  const size_t perB = (size_t)gc.n * gc.n * gc.p * es;  // bytes of factors per problem
-  const size_t xB[3] = {(size_t)gc.n * 16, (size_t)gc.n * es, (size_t)gc.n * 8};
-  const bool wantZ = gc.wantZ && Z;
-  // One CTA works on one problem (for seconds at the larger orders), so a launch should carry at
-  // least two problems per SM; beyond that, 512 MiB of factors per launch keeps the copies of one
-  // chunk under the kernels of the others.  The cap keeps the slots inside device memory.
-  const bool wantZ0 = gc.wantZ && Z;
-  long long chunk = std::max<long long>(1, (512LL << 20) / (long long)perB);
+// Chunk sizes of the generalized paths for `count` problems of `per` bytes of factors and
+// `dev_per` bytes of device buffers.  One CTA works on one problem (for seconds at the larger
+// orders), so a launch should carry at least two problems per SM; beyond that, 512 MiB of factors
+// per launch keeps the copies of one chunk under the kernels of the others.  The cap keeps the
+// slots inside device memory.
+int plan_gen_chunks(const Device& dev, long long count, size_t per, size_t dev_per, std::vector<long long>& chunks) {
+  long long chunk = std::max<long long>(1, (512LL << 20) / (long long)per);
   const long long wave = 2LL * dev.sm_count;  // resident problems per launch in global-memory mode
   chunk = (chunk + wave - 1) / wave * wave;   // whole waves: no half-empty tail inside a launch
-  {
-    size_t free_b = 0, total_b = 0;
-    PSD_SHARD_CUDA(cudaMemGetInfo(&free_b, &total_b));
-    const size_t per_problem = perB * (wantZ0 ? 2 : 1) + (xB[0] + xB[1] + xB[2]) + 64;
-    const long long cap = (long long)((total_b / 2) / kSlotsPerDevice / per_problem);
-    chunk = std::max<long long>(1, std::min(chunk, cap));
-  }
-  chunk = std::min(chunk, count);
-  // chunks above this size are copied straight from / to pageable memory (no pinned staging copy)
-  const size_t kStageLimit = 1ULL << 30;
-  int si = 0;
-  // results of a staged (pageable) chunk that still sit in a slot's pinned buffers: copied out when
-  // the slot is drained, so that the host copies overlap the device work of the other slots
-  struct Pending {
-    bool any = false;
-    char *dstA = nullptr, *dstZ = nullptr, *dstX[3] = {nullptr, nullptr, nullptr};
-    int32_t* dstInfo = nullptr;
-    size_t bytesA = 0, bytesX[3] = {0, 0, 0}, bytesInfo = 0;
-  } pend[kSlotsPerDevice];
-  auto flush = [&](int k) {
-    Pending& q = pend[k];
-    if (!q.any) return;
-    Slot& s = dev.slots[k];
-    if (q.dstA) std::memcpy(q.dstA, s.hA, q.bytesA);
-    if (q.dstZ) std::memcpy(q.dstZ, s.hZ, q.bytesA);
-    for (int t = 0; t < 3; t++)
-      if (q.dstX[t]) std::memcpy(q.dstX[t], s.hX[t], q.bytesX[t]);
-    if (q.dstInfo) std::memcpy(q.dstInfo, s.hInfo, q.bytesInfo);
-    q = Pending();
-  };
-  for (long long off = 0; off < count; off += chunk, si = (si + 1) % kSlotsPerDevice) {
-    const long long nb = std::min(chunk, count - off);
-    Slot& s = dev.slots[si];
-    if (!s.stream) PSD_SHARD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-    PSD_SHARD_CUDA(cudaStreamSynchronize(s.stream));
-    flush(si);
-    int e;
-    const size_t bytesA = nb * perB;
-    if ((e = ensure_dev(s.dA, s.capA, bytesA))) return drain_slots(dev, e);
-    if (wantZ && (e = ensure_dev(s.dZ, s.capZ, bytesA))) return drain_slots(dev, e);
-    for (int k = 0; k < 3; k++)
-      if ((e = ensure_dev(s.dX[k], s.capX[k], nb * xB[k]))) return drain_slots(dev, e);
-    if ((e = ensure_dev(s.dInfo, s.capInfo, nb * sizeof(int32_t)))) return drain_slots(dev, e);
-    char* srcA = A + (size_t)(first + off) * perB;
-    const bool direct = pinned || bytesA > kStageLimit;
-    if (direct) {
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.dA, srcA, bytesA, cudaMemcpyHostToDevice, s.stream));
-    } else {
-      if ((e = ensure_pinned(s.hA, s.hcapA, bytesA))) return drain_slots(dev, e);
-      std::memcpy(s.hA, srcA, bytesA);
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.dA, s.hA, bytesA, cudaMemcpyHostToDevice, s.stream));
-    }
-    *bytes_h2d += (int64_t)bytesA;
-    e = launch_gen(h, dev, s, s.stream, gc, nb, s.dA, wantZ ? s.dZ : nullptr, s.dX[0], s.dX[1],
-                   (long long*)s.dX[2], s.dInfo);
-    if (e) return drain_slots(dev, e);
-    char* dstZ = wantZ ? Z + (size_t)(first + off) * perB : nullptr;
-    const bool ev = !gc.reduce_only;
-    char* dstX[3] = {ev ? alpha + (size_t)(first + off) * xB[0] : nullptr, ev ? beta + (size_t)(first + off) * xB[1] : nullptr,
-                     ev ? (char*)scale + (size_t)(first + off) * xB[2] : nullptr};
-    int32_t* dstInfo = ev ? info + (first + off) : nullptr;
-    const size_t bytesInfo = nb * sizeof(int32_t);
-    if (direct) {
-      if (gc.wantT) PSD_SHARD_CUDA(cudaMemcpyAsync(srcA, s.dA, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      if (wantZ) PSD_SHARD_CUDA(cudaMemcpyAsync(dstZ, s.dZ, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      for (int k = 0; k < 3 && ev; k++)
-        PSD_SHARD_CUDA(cudaMemcpyAsync(dstX[k], s.dX[k], nb * xB[k], cudaMemcpyDeviceToHost, s.stream));
-      if (ev) PSD_SHARD_CUDA(cudaMemcpyAsync(dstInfo, s.dInfo, bytesInfo, cudaMemcpyDeviceToHost, s.stream));
-    } else {
-      if (wantZ && (e = ensure_pinned(s.hZ, s.hcapZ, bytesA))) return drain_slots(dev, e);
-      for (int k = 0; k < 3; k++)
-        if ((e = ensure_pinned(s.hX[k], s.hcapX[k], nb * xB[k]))) return drain_slots(dev, e);
-      if ((e = ensure_pinned(s.hInfo, s.hcapInfo, bytesInfo))) return drain_slots(dev, e);
-      if (gc.wantT) PSD_SHARD_CUDA(cudaMemcpyAsync(s.hA, s.dA, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      if (wantZ) PSD_SHARD_CUDA(cudaMemcpyAsync(s.hZ, s.dZ, bytesA, cudaMemcpyDeviceToHost, s.stream));
-      for (int k = 0; k < 3; k++)
-        PSD_SHARD_CUDA(cudaMemcpyAsync(s.hX[k], s.dX[k], nb * xB[k], cudaMemcpyDeviceToHost, s.stream));
-      PSD_SHARD_CUDA(cudaMemcpyAsync(s.hInfo, s.dInfo, bytesInfo, cudaMemcpyDeviceToHost, s.stream));
-      Pending& q = pend[si];
-      q.any = true;
-      q.dstA = gc.wantT ? srcA : nullptr;
-      q.dstZ = wantZ ? dstZ : nullptr;
-      for (int k = 0; k < 3; k++) { q.dstX[k] = ev ? dstX[k] : nullptr; q.bytesX[k] = nb * xB[k]; }
-      q.dstInfo = ev ? dstInfo : nullptr;
-      q.bytesA = bytesA; q.bytesInfo = bytesInfo;
-    }
-    *bytes_d2h += (int64_t)((gc.wantT ? bytesA : 0) + (wantZ ? bytesA : 0) + nb * (xB[0] + xB[1] + xB[2]) + bytesInfo);
-  }
-  for (int k = 0; k < kSlotsPerDevice; k++)
-    if (dev.slots[k].stream) {
-      PSD_SHARD_CUDA(cudaStreamSynchronize(dev.slots[k].stream));
-      flush(k);
-    }
+  size_t free_b = 0, total_b = 0;
+  PSD_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  const long long cap = (long long)((total_b / 2) / kSlotsPerDevice / dev_per);
+  chunk = std::min(std::max<long long>(1, std::min(chunk, cap)), count);
+  for (long long off = 0; off < count; off += chunk) chunks.push_back(std::min(chunk, count - off));
   return PSD_OK;
 }
 
@@ -1099,38 +1025,31 @@ int run_gen_host(psd_handle_t h, const GenCall& gc, int64_t batch, void* A, void
   // leftmost factor after orientation must have S = true (generalized.jl:140, rgeneralized.jl:37)
   if (!gc.S[gc.left ? gc.p - 1 : 0]) return fail(PSD_ERR_SIGNATURE, "The leftmost entry in S must be true");
   if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
-  std::lock_guard<std::mutex> lock(h->mu);
-  for (auto& s : h->stats) s = 0;
-  if (batch == 0) return PSD_OK;
-  const bool pinned = is_pinned(A) && is_pinned(Z) && is_pinned(alpha) && is_pinned(beta) && is_pinned(scale) &&
-                      is_pinned(info);
-  const int nd = (int)h->devs.size();
-  std::vector<int> codes(nd, PSD_OK);
-  std::vector<std::string> msgs(nd);
-  std::vector<int64_t> h2d(nd, 0), d2h(nd, 0);
-  auto t0 = std::chrono::steady_clock::now();
-  auto work = [&](int d) {
-    const long long lo = batch * d / nd, hi = batch * (d + 1) / nd;
-    codes[d] = run_gen_shard(h, h->devs[d], gc, lo, hi - lo, (char*)A, (char*)Z, (char*)alpha, (char*)beta, scale,
-                             info, pinned, &h2d[d], &d2h[d]);
-    if (codes[d]) msgs[d] = g_err;
-  };
-  if (nd == 1) {
-    work(0);
-  } else {
-    std::vector<std::thread> th;
-    for (int d = 0; d < nd; d++) th.emplace_back(work, d);
-    for (auto& t : th) t.join();
-  }
-  auto t1 = std::chrono::steady_clock::now();
-  for (int d = 0; d < nd; d++) {
-    h->stats[3] += h2d[d];
-    h->stats[4] += d2h[d];
-  }
-  h->stats[5] = std::chrono::duration_cast<std::chrono::microseconds>(t1 - t0).count();
-  for (int d = 0; d < nd; d++)
-    if (codes[d]) return fail(codes[d], msgs[d]);
-  return PSD_OK;
+  const size_t es = gen_elem(gc);
+  const size_t per = (size_t)gc.n * gc.n * gc.p * es;  // bytes of factors per problem
+  const size_t xB[3] = {(size_t)gc.n * 16, (size_t)gc.n * es, (size_t)gc.n * 8};  // alpha, beta, alphascale
+  const bool wantZ = gc.wantZ && Z;
+  return run_host(h, batch, {A, Z, alpha, beta, scale, info}, [&](Device& dev, long long first, long long count,
+                                                                  bool pinned, int64_t* bytes_h2d, int64_t* bytes_d2h) {
+    std::vector<long long> chunks;
+    if (int e = plan_gen_chunks(dev, count, per, per * (wantZ ? 2 : 1) + (xB[0] + xB[1] + xB[2]) + 64, chunks))
+      return e;
+    std::vector<HostArray> in{{(char*)A, per, kFactors}}, out;
+    if (gc.wantT) out.push_back({(char*)A, per, kFactors});
+    if (wantZ) out.push_back({(char*)Z, per, kZ});
+    if (!gc.reduce_only) {
+      out.push_back({(char*)alpha, xB[0], kVal0});
+      out.push_back({(char*)beta, xB[1], kVal1});
+      out.push_back({(char*)scale, xB[2], kVal2});
+    }
+    // the reduction-only kernel writes info as well, which the call does not return
+    out.push_back({gc.reduce_only ? nullptr : (char*)info, sizeof(int32_t), kInfo});
+    auto launch = [&](Slot& s, long long nb, void* const* d) {
+      return launch_gen(h, dev, s, s.stream, gc, nb, d[kFactors], d[kZ], d[kVal0], d[kVal1], (long long*)d[kVal2],
+                        (int32_t*)d[kInfo]);
+    };
+    return run_shard(dev, first, chunks, pinned, in, out, launch, bytes_h2d, bytes_d2h);
+  });
 }
 
 }  // namespace
@@ -1196,17 +1115,19 @@ int psd_destroy(psd_handle_t h) {
         cudaStreamSynchronize(s.stream);
         cudaStreamDestroy(s.stream);
       }
-      cudaFree(s.dA); cudaFree(s.dZ); cudaFree(s.dEig); cudaFree(s.dInfo);
+      for (int k = 0; k < kRoles; k++) {
+        cudaFree(s.dBuf[k]);
+        cudaFreeHost(s.hBuf[k]);
+      }
       cudaFree(s.dCounter); cudaFree(s.dScratch); cudaFree(s.dPacked); cudaFree(s.dS);
       for (int k = 0; k < 8; k++) cudaFree(s.dPk[k]);
       cudaFree(s.dPhaseCtr);
       cudaFree(s.dProf);
       psd::ms::ws_destroy(s.ms);
       for (int k = 0; k < 3; k++) {
-        cudaFree(s.dX[k]);
-        cudaFreeHost(s.hX[k]);
+        cudaFree(s.dArg[k]);
+        cudaFree(s.dTeam[k]);
       }
-      cudaFreeHost(s.hA); cudaFreeHost(s.hZ); cudaFreeHost(s.hEig); cudaFreeHost(s.hInfo);
     };
     for (auto& s : d.slots) freeSlot(s);
     freeSlot(d.user);
@@ -1249,11 +1170,9 @@ int psd_rcheckpsd_batched(psd_handle_t h, int n, int p, int64_t batch, int orien
   if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
   std::lock_guard<std::mutex> lock(h->mu);
   if (batch == 0) return PSD_OK;
+  if (int e = use_slot0(h)) return e;
   Device& dev = h->devs[0];
-  PSD_CUDA(cudaSetDevice(dev.ordinal));
   Slot& s = dev.slots[0];
-  if (!s.stream) PSD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-  PSD_CUDA(cudaStreamSynchronize(s.stream));
   const size_t per = (size_t)n * n * p;
   // a diagnostic, not a hot path: plain chunks of at most ~1 GiB per array, synchronous copies
   const long long chunk = std::max<long long>(1, std::min<long long>(batch, (1LL << 30) / (long long)(per * sizeof(double))));
@@ -1323,27 +1242,25 @@ int psd_rphess_packed_batched(psd_handle_t h, int n, int p, int64_t batch, doubl
   if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
   std::lock_guard<std::mutex> lock(h->mu);
   if (batch == 0) return PSD_OK;
+  if (int e = use_slot0(h)) return e;
   Device& dev = h->devs[0];
-  PSD_CUDA(cudaSetDevice(dev.ordinal));
   Slot& s = dev.slots[0];
-  if (!s.stream) PSD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-  PSD_CUDA(cudaStreamSynchronize(s.stream));
   const size_t per = (size_t)n * n * p;
   const long long chunk = std::max<long long>(1, std::min<long long>(batch, (1LL << 30) / (long long)(per * sizeof(double))));
   int e;
-  if ((e = ensure_dev(s.dA, s.capA, chunk * per * sizeof(double)))) return e;
-  if ((e = ensure_dev(s.dEig, s.capEig, std::max<size_t>((size_t)chunk * p * n, (size_t)chunk * 2 * n) * sizeof(double)))) return e;
-  if ((e = ensure_dev(s.dInfo, s.capInfo, chunk * sizeof(int32_t)))) return e;
+  if ((e = ensure_dev(s.dArg[0], s.capArg[0], chunk * per * sizeof(double)))) return e;
+  if ((e = ensure_dev(s.dArg[1], s.capArg[1], std::max<size_t>((size_t)chunk * p * n, (size_t)chunk * 2 * n) * sizeof(double)))) return e;
+  if ((e = ensure_dev(s.dArg[2], s.capArg[2], chunk * sizeof(int32_t)))) return e;
   RealCall rc{n, p, 0, 1, 0, 30, 1, 0};
   for (long long off = 0; off < batch; off += chunk) {
     const long long nb = std::min(chunk, batch - off);
-    PSD_CUDA(cudaMemcpyAsync(s.dA, A + (size_t)off * per, nb * per * sizeof(double), cudaMemcpyHostToDevice, s.stream));
-    s.curTau = s.dEig;  // (the eigenvalue buffer is unused by a reduction-only launch)
-    e = launch_real(h, dev, s, s.stream, rc, nb, s.dA, nullptr, nullptr, s.dInfo);
+    PSD_CUDA(cudaMemcpyAsync(s.dArg[0], A + (size_t)off * per, nb * per * sizeof(double), cudaMemcpyHostToDevice, s.stream));
+    s.curTau = s.dArg[1];
+    e = launch_real(h, dev, s, s.stream, rc, nb, s.dArg[0], nullptr, nullptr, (int32_t*)s.dArg[2]);
     s.curTau = nullptr;
     if (e) return e;
-    PSD_CUDA(cudaMemcpyAsync(A + (size_t)off * per, s.dA, nb * per * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
-    PSD_CUDA(cudaMemcpyAsync(tau + (size_t)off * p * n, s.dEig, nb * p * n * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
+    PSD_CUDA(cudaMemcpyAsync(A + (size_t)off * per, s.dArg[0], nb * per * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
+    PSD_CUDA(cudaMemcpyAsync(tau + (size_t)off * p * n, s.dArg[1], nb * p * n * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
     PSD_CUDA(cudaStreamSynchronize(s.stream));
   }
   return PSD_OK;
@@ -1451,24 +1368,23 @@ int psd_rphess_rowwise_batched(psd_handle_t h, int n, int extra_row, int p, int 
   std::lock_guard<std::mutex> lock(h->mu);
   for (auto& s : h->stats) s = 0;
   if (batch == 0) return PSD_OK;
+  if (int e = use_slot0(h)) return e;
   Device& dev = h->devs[0];
-  PSD_CUDA(cudaSetDevice(dev.ordinal));
   Slot& s = dev.slots[0];
-  if (!s.stream) PSD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
   const int m = n + (extra_row ? 1 : 0);
   const size_t bAp = (size_t)batch * m * n * sizeof(double);
   const size_t bA = (size_t)batch * (p - 1) * n * n * sizeof(double);
   const size_t bQ = Q ? (size_t)batch * p * qrows * n * sizeof(double) : 0;
   int e;
-  if ((e = ensure_dev(s.dA, s.capA, bAp))) return e;
-  if (bA && (e = ensure_dev(s.dZ, s.capZ, bA))) return e;
-  if (bQ && (e = ensure_dev(s.dX[0], s.capX[0], bQ))) return e;
-  PSD_CUDA(cudaMemcpyAsync(s.dA, Ap, bAp, cudaMemcpyHostToDevice, s.stream));
-  if (bA) PSD_CUDA(cudaMemcpyAsync(s.dZ, A, bA, cudaMemcpyHostToDevice, s.stream));
-  if (bQ) PSD_CUDA(cudaMemcpyAsync(s.dX[0], Q, bQ, cudaMemcpyHostToDevice, s.stream));
+  if ((e = ensure_dev(s.dArg[0], s.capArg[0], bAp))) return e;
+  if (bA && (e = ensure_dev(s.dArg[1], s.capArg[1], bA))) return e;
+  if (bQ && (e = ensure_dev(s.dArg[2], s.capArg[2], bQ))) return e;
+  PSD_CUDA(cudaMemcpyAsync(s.dArg[0], Ap, bAp, cudaMemcpyHostToDevice, s.stream));
+  if (bA) PSD_CUDA(cudaMemcpyAsync(s.dArg[1], A, bA, cudaMemcpyHostToDevice, s.stream));
+  if (bQ) PSD_CUDA(cudaMemcpyAsync(s.dArg[2], Q, bQ, cudaMemcpyHostToDevice, s.stream));
   psd::RowHessParams<double> P;
   P.n = n; P.m = m; P.p = p; P.qrows = qrows; P.batch = batch;
-  P.Ap = s.dA; P.A = bA ? s.dZ : nullptr; P.Q = bQ ? (double*)s.dX[0] : nullptr;
+  P.Ap = s.dArg[0]; P.A = bA ? s.dArg[1] : nullptr; P.Q = bQ ? s.dArg[2] : nullptr;
   const int threads = std::max(64, std::min(256, ((std::max(n, qrows) + 31) / 32) * 32));
   const int grid = (int)std::min<long long>(batch, (long long)dev.sm_count * 4);
   {
@@ -1476,9 +1392,9 @@ int psd_rphess_rowwise_batched(psd_handle_t h, int n, int extra_row, int p, int 
     psd::rowhess_kernel<double><<<grid, threads, (size_t)(n + 2) * sizeof(double), s.stream>>>(P);
   }
   PSD_CUDA(cudaGetLastError());
-  PSD_CUDA(cudaMemcpyAsync(Ap, s.dA, bAp, cudaMemcpyDeviceToHost, s.stream));
-  if (bA) PSD_CUDA(cudaMemcpyAsync(A, s.dZ, bA, cudaMemcpyDeviceToHost, s.stream));
-  if (bQ) PSD_CUDA(cudaMemcpyAsync(Q, s.dX[0], bQ, cudaMemcpyDeviceToHost, s.stream));
+  PSD_CUDA(cudaMemcpyAsync(Ap, s.dArg[0], bAp, cudaMemcpyDeviceToHost, s.stream));
+  if (bA) PSD_CUDA(cudaMemcpyAsync(A, s.dArg[1], bA, cudaMemcpyDeviceToHost, s.stream));
+  if (bQ) PSD_CUDA(cudaMemcpyAsync(Q, s.dArg[2], bQ, cudaMemcpyDeviceToHost, s.stream));
   PSD_CUDA(cudaStreamSynchronize(s.stream));
   h->stats[0] = 1;
   h->stats[2] = batch;
@@ -1493,26 +1409,25 @@ int psd_dgemm_host(psd_handle_t h, int transA, int transB, int M, int N, int K, 
   if (M < 0 || N < 0 || K < 0 || !A || !B || !C) return fail(PSD_ERR_BAD_ARG, "bad argument");
   if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
   std::lock_guard<std::mutex> lock(h->mu);
+  if (int e = use_slot0(h)) return e;
   Device& dev = h->devs[0];
-  PSD_CUDA(cudaSetDevice(dev.ordinal));
   Slot& s = dev.slots[0];
-  if (!s.stream) PSD_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
   const size_t bA = (size_t)lda * (transA ? M : K) * 8, bB = (size_t)ldb * (transB ? K : N) * 8;
   const size_t bC = (size_t)ldc * N * 8;
   int e;
-  if ((e = ensure_dev(s.dA, s.capA, bA))) return e;
-  if ((e = ensure_dev(s.dZ, s.capZ, bB))) return e;
-  if ((e = ensure_dev(s.dX[0], s.capX[0], bC))) return e;
-  PSD_CUDA(cudaMemcpyAsync(s.dA, A, bA, cudaMemcpyHostToDevice, s.stream));
-  PSD_CUDA(cudaMemcpyAsync(s.dZ, B, bB, cudaMemcpyHostToDevice, s.stream));
-  PSD_CUDA(cudaMemcpyAsync(s.dX[0], C, bC, cudaMemcpyHostToDevice, s.stream));
+  if ((e = ensure_dev(s.dArg[0], s.capArg[0], bA))) return e;
+  if ((e = ensure_dev(s.dArg[1], s.capArg[1], bB))) return e;
+  if ((e = ensure_dev(s.dArg[2], s.capArg[2], bC))) return e;
+  PSD_CUDA(cudaMemcpyAsync(s.dArg[0], A, bA, cudaMemcpyHostToDevice, s.stream));
+  PSD_CUDA(cudaMemcpyAsync(s.dArg[1], B, bB, cudaMemcpyHostToDevice, s.stream));
+  PSD_CUDA(cudaMemcpyAsync(s.dArg[2], C, bC, cudaMemcpyHostToDevice, s.stream));
   psd::GemmArgs g;
   g.M = M; g.N = N; g.K = K;
-  g.A = s.dA; g.rsA = transA ? lda : 1; g.csA = transA ? 1 : lda;
-  g.B = s.dZ; g.rsB = transB ? ldb : 1; g.csB = transB ? 1 : ldb;
-  g.C = (double*)s.dX[0]; g.ldc = ldc; g.alpha = alpha; g.beta = beta; g.splitK = 1;
+  g.A = s.dArg[0]; g.rsA = transA ? lda : 1; g.csA = transA ? 1 : lda;
+  g.B = s.dArg[1]; g.rsB = transB ? ldb : 1; g.csB = transB ? 1 : ldb;
+  g.C = s.dArg[2]; g.ldc = ldc; g.alpha = alpha; g.beta = beta; g.splitK = 1;
   PSD_CUDA(psd::dgemm_launch(s.stream, dev.sm_count, g));
-  PSD_CUDA(cudaMemcpyAsync(C, s.dX[0], bC, cudaMemcpyDeviceToHost, s.stream));
+  PSD_CUDA(cudaMemcpyAsync(C, s.dArg[2], bC, cudaMemcpyDeviceToHost, s.stream));
   PSD_CUDA(cudaStreamSynchronize(s.stream));
   if (reps > 0 && ms) {
     cudaEvent_t e0, e1;
