@@ -15,7 +15,10 @@
 //    previous link's reflectors, so the serial dependency chain contains no shuffle and no
 //    shared-memory access; the 3-reflector of link t and the 2-reflector of link t-1 are
 //    computed in the same slot (two independent dependency chains = ILP), and the row/column
-//    updates of link t-1 ("bulk") are applied lane-parallel in that slot as well;
+//    updates of link t-1 ("bulk") are applied lane-parallel in that slot as well; with the
+//    period fixed at compile time (p >= 4, the headline instantiation) the bulk runs two links
+//    behind instead, so that it no longer waits for the 2-reflector of the same slot
+//    (sweep_lag2);
 //  * reflectors are kept un-normalised, H = I + g u u^T with g = -2/(u^T u): one rsqrt and
 //    one reciprocal (MUFU seed + Newton steps) instead of dlarfg's sqrt + three divisions
 //    (householder.jl:66-108); orthogonality of H depends only on g, not on the accuracy of
@@ -30,6 +33,8 @@
 //
 // Indices in this file are 0-based.
 #pragma once
+#include <type_traits>
+
 #include "psd_device.cuh"
 
 namespace psd {
@@ -303,11 +308,188 @@ PSD_DEV void col_pass_h1(double* sm, int oc1, int q, int r, int i, int l, bool c
   if ((reg || src) && c2) sm[a + 2] = a2;
 }
 
+// Both reflectors of one link, kept until its row/column passes ("bulk") run.  The H1 link has
+// no 2-reflector; its bulk uses u, g and beta only.
+struct LinkRefl {
+  double u0, u1, u2, g, beta;
+  double b0, b1, bh, beta2;
+};
+
+// 3x3 diagonal block of a link, prefetched one slot before its A part.
+struct Blk {
+  double x00, x01, x02, x10, x11, x12, x22;
+};
+
+// Block of triangular factor at `hb`, rows/columns k..k+2 (k..k+1 when C2 is false).
+template <bool C2>
+PSD_DEV Blk prefetch_tri(const double* sm, int hb, int t1a, int t1b, int t1c, int k) {
+  Blk y;
+  y.x00 = sm[hb + t1a + k];
+  y.x01 = sm[hb + t1b + k];
+  y.x10 = 0.0;
+  y.x11 = sm[hb + t1b + k + 1];
+  y.x02 = C2 ? sm[hb + t1c + k] : 0.0;
+  y.x12 = C2 ? sm[hb + t1c + k + 1] : 0.0;
+  y.x22 = C2 ? sm[hb + t1c + k + 2] : 0.0;
+  return y;
+}
+
+// Block of the link H1(k+1): rows k+1..k+3, columns k..k+2 of H1 (only needed while k+2 <= i).
+PSD_DEV Blk prefetch_h1(const double* sm, int t3a, int t3b, int t3c, int k, int i) {
+  Blk y;
+  const bool r3 = (k + 3 <= i);
+  y.x00 = sm[t3a + k + 1];
+  y.x01 = sm[t3b + k + 1];
+  y.x02 = sm[t3c + k + 1];
+  y.x10 = sm[t3a + k + 2];
+  y.x11 = sm[t3b + k + 2];
+  y.x12 = sm[t3c + k + 2];
+  y.x22 = sm[t3c + (r3 ? k + 3 : k + 1)];
+  y.x22 = r3 ? y.x22 : 0.0;
+  return y;
+}
+
+PSD_DEV void set_block(ChainState& c, const Blk& y) {
+  c.x00 = y.x00; c.x01 = y.x01; c.x02 = y.x02; c.x10 = y.x10; c.x11 = y.x11; c.x12 = y.x12;
+  c.x22 = y.x22;
+}
+
+// Double-shift sweep over the window l..i with the bulk lagging TWO links behind the chain, for
+// a period P >= 4 fixed at compile time.  The slot of link t (chain order H1(k), factor P, ...,
+// factor 2, H1(k+1), ...) runs three independent streams:
+//   * the A part and 3-reflector of link t (the loop-carried chain);
+//   * the B part (2-reflector) of link t-1;
+//   * the bulk of link t-2: column pass on its matrix M(t-2), row pass on M(t-1).
+// The slot also prefetches the block of link t+1 from M(t+1) before its bulk.  Lag rule: compared
+// with the one-link lag of the generic sweep, the only update that moves behind a prefetch is the
+// bulk of link t-2 behind the prefetch of M(t+1) in slot t.  It writes M(t-2) and M(t-1), and links
+// P apart share a matrix, so with P >= 4 it touches no prefetched entry:
+//   * factor links: the block of factor j at step k still has pending only the row pass of link
+//     t (folded by chain_A / chain_B, as before); the passes of step k-1 on factor j, the column
+//     pass of factor j (k-1) (rows k-1..k+1) and the row pass of factor j+1 (k-1), or of H1(k-1)
+//     for j = P (columns k-1..k+1), ran P-3 and P-2 slots before the prefetch;
+//   * the H1 link: the block of H1(k+1) is read in the factor-2 slot of step k (slot P-1 of the
+//     step), after the column pass of H1(k) (slot 2, needs P - 1 > 2) and the row pass of
+//     factor 2 (k-1) (slot 1); the row pass of factor 2 (k) is folded by chain_A / chain_B.
+// At P = 3 the column pass of M(t-2) = M(t+1) would hit rows k, k+1 of the prefetched block, so
+// smaller periods keep the generic sweep.  Every stored element and every chain value therefore
+// gets the same operations as in the generic sweep; only their order across slots differs.
+// The factor loop is fully unrolled (prefetch sources and packed offsets are resolved per slot)
+// and the last step of the sweep (k = i-1, the only one with k+2 > i) has its own instantiation.
+template <bool SAFE, int P>
+PSD_DEV void sweep_lag2(double* sm, const int szh1, const int sj, const int l, const int i,
+                        const int r, const int ocj, const int oc1, const double v0, const double v1,
+                        const double v2, bool& bad) {
+  static_assert(P >= 4, "the two-link lag needs a period of at least 4");
+  ChainState c;
+  c.c0 = c.c1 = c.h = 0.0;
+  LinkRefl d;  // reflectors of the link whose bulk is pending (link t-2 at the start of slot t)
+  int t1a = pk_off(1, l), t1b = pk_off(1, l + 1), t1c = pk_off(1, l + 2);
+  int t3a = pk_off(3, l), t3b = pk_off(3, l + 1), t3c = pk_off(3, l + 2);
+  // previous step's offsets: the bulks of factors 3 and 2 run in the first two slots of a step
+  int p1a = 0, p1b = 0, p1c = 0, p3a = 0, p3b = 0, p3c = 0;
+  auto step = [&](const int k, auto c2tag) {
+    constexpr bool C2 = decltype(c2tag)::value;  // k + 2 <= i
+    const int rm2 = C2 ? k + 2 : k + 1;           // min(k + 2, i)
+    double s0, s1, s2, m01, m02, m11, m12, m21, m22, nu0, ng, nbeta;
+    Blk y;
+    // =============== slot H1(k): bulk of factor 3 (k-1), B part of factor 2 (k-1) ===============
+    __syncwarp();
+    y = prefetch_tri<C2>(sm, szh1 + (P - 2) * sj, t1a, t1b, t1c, k);
+    if (k > l) {
+      double b0, b1, bh;
+      const double beta2 = chain_B<SAFE>(c, b0, b1, bh, bad);
+      row_pass<1, true>(sm, szh1, p1a, p1b, p1c, k - 1, r, l, k + 1, true, d.u0, d.u1, d.u2, d.g,
+                        d.b0, d.b1, d.bh);
+      col_pass_tri(sm, szh1 + sj, ocj, k - 1, r, i, true, d.u0, d.u1, d.u2, d.g, d.beta, d.b0, d.b1,
+                   d.bh, d.beta2);
+      chain_A(c, s0, s1, s2, m01, m02, m11, m12, m21, m22);
+      d = LinkRefl{c.u0, c.u1, c.u2, c.g, c.beta, b0, b1, bh, beta2};
+    } else {
+      s0 = v0; s1 = v1; s2 = v2;
+    }
+    nbeta = refl_u<3, SAFE>(s0, s1, s2, nu0, ng, bad);
+    set_block(c, y);
+    c.u0 = nu0; c.u1 = s1; c.u2 = s2; c.g = ng; c.beta = nbeta;
+    // =============== slot factor P: bulk of factor 2 (k-1) ===============
+    __syncwarp();
+    y = prefetch_tri<C2>(sm, szh1 + (P - 3) * sj, t1a, t1b, t1c, k);
+    if (k > l) {
+      row_pass<3, true>(sm, 0, p3a, p3b, p3c, k - 1, r, l, rm2, true, d.u0, d.u1, d.u2, d.g, d.b0,
+                        d.b1, d.bh);
+      col_pass_tri(sm, szh1, ocj, k - 1, r, i, true, d.u0, d.u1, d.u2, d.g, d.beta, d.b0, d.b1, d.bh,
+                   d.beta2);
+    }
+    chain_A(c, s0, s1, s2, m01, m02, m11, m12, m21, m22);
+    nbeta = refl_u<3, SAFE>(s0, s1, s2, nu0, ng, bad);
+    d.u0 = c.u0; d.u1 = c.u1; d.u2 = c.u2; d.g = c.g; d.beta = c.beta;  // H1(k)
+    set_block(c, y);
+    c.c0 = 0.0; c.c1 = 0.0; c.h = 0.0;  // the H1 link has no 2-reflector
+    c.u0 = nu0; c.u1 = s1; c.u2 = s2; c.g = ng; c.beta = nbeta;
+    c.n01 = m01; c.n02 = m02; c.n11 = m11; c.n12 = m12; c.n21 = m21; c.n22 = m22;
+    // ====== slots factor P-1 .. 2: B part of factor j+1, bulk of factor j+2 (H1(k) for j = P-1) ======
+#pragma unroll
+    for (int j = P - 1; j >= 2; j--) {
+      __syncwarp();
+      if (j > 2)
+        y = prefetch_tri<C2>(sm, szh1 + (j - 3) * sj, t1a, t1b, t1c, k);
+      else if (C2)
+        y = prefetch_h1(sm, t3a, t3b, t3c, k, i);
+      double b0, b1, bh;
+      const double beta2 = chain_B<SAFE>(c, b0, b1, bh, bad);
+      if (j == P - 1) {
+        row_pass<1, false>(sm, szh1 + (P - 2) * sj, t1a, t1b, t1c, k, r, l, rm2, C2, d.u0, d.u1, d.u2,
+                           d.g, 0.0, 0.0, 0.0);
+        col_pass_h1(sm, oc1, k, r, i, l, C2, d.u0, d.u1, d.u2, d.g, d.beta);
+      } else {
+        row_pass<1, true>(sm, szh1 + (j - 1) * sj, t1a, t1b, t1c, k, r, l, rm2, C2, d.u0, d.u1, d.u2,
+                          d.g, d.b0, d.b1, d.bh);
+        col_pass_tri(sm, szh1 + j * sj, ocj, k, r, i, C2, d.u0, d.u1, d.u2, d.g, d.beta, d.b0, d.b1,
+                     d.bh, d.beta2);
+      }
+      chain_A(c, s0, s1, s2, m01, m02, m11, m12, m21, m22);
+      nbeta = refl_u<3, SAFE>(s0, s1, s2, nu0, ng, bad);
+      d = LinkRefl{c.u0, c.u1, c.u2, c.g, c.beta, b0, b1, bh, beta2};  // factor j+1
+      if (j > 2 || C2) set_block(c, y);
+      c.c0 = b0; c.c1 = b1; c.h = bh;
+      c.u0 = nu0; c.u1 = s1; c.u2 = s2; c.g = ng; c.beta = nbeta;
+      c.n01 = m01; c.n02 = m02; c.n11 = m11; c.n12 = m12; c.n21 = m21; c.n22 = m22;
+    }
+    p1a = t1a; p1b = t1b; p1c = t1c;
+    p3a = t3a; p3b = t3b; p3c = t3c;
+    t1a = t1b; t1b = t1c; t1c += (k + 3) + 1;
+    t3a = t3b; t3b = t3c; t3c += (k + 3) + 3;
+  };
+  for (int k = l; k < i - 1; k++) step(k, std::true_type{});
+  step(i - 1, std::false_type{});
+  // flush, two drained links: B part of factor 2 and bulk of factor 3 at k = i-1 ...
+  {
+    __syncwarp();
+    double b0, b1, bh;
+    const double beta2 = chain_B<SAFE>(c, b0, b1, bh, bad);
+    row_pass<1, true>(sm, szh1, p1a, p1b, p1c, i - 1, r, l, i, false, d.u0, d.u1, d.u2, d.g, d.b0,
+                      d.b1, d.bh);
+    col_pass_tri(sm, szh1 + sj, ocj, i - 1, r, i, false, d.u0, d.u1, d.u2, d.g, d.beta, d.b0, d.b1,
+                 d.bh, d.beta2);
+    d = LinkRefl{c.u0, c.u1, c.u2, c.g, c.beta, b0, b1, bh, beta2};
+  }
+  // ... then the bulk of factor 2 at k = i-1
+  {
+    __syncwarp();
+    row_pass<3, true>(sm, 0, p3a, p3b, p3c, i - 1, r, l, i, false, d.u0, d.u1, d.u2, d.g, d.b0, d.b1,
+                      d.bh);
+    col_pass_tri(sm, szh1, ocj, i - 1, r, i, false, d.u0, d.u1, d.u2, d.g, d.beta, d.b0, d.b1, d.bh,
+                 d.beta2);
+  }
+}
+
 // Result of one problem: info >= 0 as documented; kNeedSafe = magnitudes left the range the
 // branch-free reflector handles, redo with SAFE = true.
 constexpr int kNeedSafe = -12345;
 
-template <bool SAFE>
+// LAG2P > 0: the period is LAG2P (>= 4) and the sweep is sweep_lag2<SAFE, LAG2P>; 0: the generic
+// sweep below, for any p >= 3 at run time.
+template <bool SAFE, int LAG2P>
 __device__ __forceinline__ int rpqr_problem(double* sm, const int n, const int p, const int i0,
                                             const int ml0, const int stop, const int lane,
                                             double& lre_out, double& lim_out, int& niter_out,
@@ -466,7 +648,9 @@ __device__ __forceinline__ int rpqr_problem(double* sm, const int n, const int p
           }
 
           // ---- double-shift sweep restricted to the window l..i (:806-886) ----
-          {
+          if constexpr (LAG2P > 0) {
+            sweep_lag2<SAFE, LAG2P>(sm, szh1, sj, l, i, r, ocj, oc1, v0, v1, v2, bad);
+          } else {
             ChainState c;
             c.c0 = c.c1 = c.h = 0.0;
             // packed offsets of columns k, k+1, k+2 in both layouts, kept incrementally:
@@ -657,6 +841,7 @@ template <int NN, int PP>
 __device__ __forceinline__ void rpqr_eig32_body(const EigParams& P) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int n = NN ? NN : P.n, p = PP ? PP : P.p;
+  constexpr int kLag2P = (PP >= 4) ? PP : 0;  // compile-time period >= 4: sweep_lag2
   const int psize = pk_problem_size(n, p);
   const int stop = P.stop;
   double* sm = psd_smem_eig + (size_t)warp * psize;  // H1 at 0, factor j at szh1 + (j-2)*sj
@@ -687,13 +872,13 @@ __device__ __forceinline__ void rpqr_eig32_body(const EigParams& P) {
     double lre, lim;
     int niter, i_end, ml_end;
     int info = P.force_safe ? kNeedSafe
-                            : rpqr_problem<false>(sm, n, p, i0, ml0, stop, lane, lre, lim, niter, i_end, ml_end);
+                            : rpqr_problem<false, kLag2P>(sm, n, p, i0, ml0, stop, lane, lre, lim, niter, i_end, ml_end);
     if (info == kNeedSafe) {
       // badly scaled problem: redo this phase with the exactly-rescaling reflector
       __syncwarp();
       for (int e = lane; e < psize; e += 32) sm[e] = src[e];
       __syncwarp();
-      info = rpqr_problem<true>(sm, n, p, i0, ml0, stop, lane, lre, lim, niter, i_end, ml_end);
+      info = rpqr_problem<true, kLag2P>(sm, n, p, i0, ml0, stop, lane, lre, lim, niter, i_end, ml_end);
     }
     // eigenvalues found in this phase: indices i_end+1 .. i0 (all of 0..i0 after a failure, as the
     // single-phase kernel reports them)
@@ -732,6 +917,9 @@ __device__ __forceinline__ void rpqr_eig32_body(const EigParams& P) {
 }
 
 
+// At most 256 threads per CTA leaves ptxas up to 255 registers.  The <32,8> instantiation uses
+// 254 (no spills): its order-32 phase is held to 6 warps per SM by shared memory, and 6 warps
+// of 256 registers fit the register file with room to spare.
 template <int NN, int PP>
 __global__ void __launch_bounds__(256) rpqr_eig32_kernel_t(EigParams P) {
   rpqr_eig32_body<NN, PP>(P);
