@@ -82,6 +82,8 @@ struct Slot {
   unsigned long long* dPhaseCtr = nullptr;  // work counters of the phase launches
   unsigned char* dS = nullptr;  // generalized paths: the signature
   size_t capS = 0;
+  int* dPexp = nullptr;  // generalized paths: exponents of the factor normalisation, p per CTA
+  size_t capPexp = 0;
   psd::ms::Workspace* ms = nullptr;  // large-N multishift iteration (psd_ms.cu)
   void* dTeam[3] = {};  // team iteration scratch: alpha, beta, alphascale
   size_t capTeam[3] = {};
@@ -979,6 +981,8 @@ int launch_gen_t(psd_handle_s* h, Device& dev, Slot& aux, cudaStream_t stream, c
   PSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
   if (occ < 1) return fail(PSD_ERR_UNSUPPORTED, "kernel does not fit on an SM");
   const int grid = (int)std::max(1LL, std::min((long long)occ * dev.sm_count, batch));
+  if ((e = ensure_dev(aux.dPexp, aux.capPexp, (size_t)grid * p * sizeof(int)))) return e;
+  P.pexp = aux.dPexp;
   {
     ScopedKernelTimer tm(h, dev, stream, 1);
     kern<<<grid, threads, smem, stream>>>(P);
@@ -1119,7 +1123,7 @@ int psd_destroy(psd_handle_t h) {
         cudaFree(s.dBuf[k]);
         cudaFreeHost(s.hBuf[k]);
       }
-      cudaFree(s.dCounter); cudaFree(s.dScratch); cudaFree(s.dPacked); cudaFree(s.dS);
+      cudaFree(s.dCounter); cudaFree(s.dScratch); cudaFree(s.dPacked); cudaFree(s.dS); cudaFree(s.dPexp);
       for (int k = 0; k < 8; k++) cudaFree(s.dPk[k]);
       cudaFree(s.dPhaseCtr);
       cudaFree(s.dProf);

@@ -39,6 +39,8 @@ struct GpqzParams {
   int deep;                 // use the deep (table-driven, single-pass) rotation chases
   int debug;                // print a phase breakdown (cycles) for the problems of CTA 0
   unsigned long long* counter;
+  int* pexp = nullptr;      // [gridDim.x][p] gpschur_kernel: power-of-two exponents of the factors of the
+                            // problem a CTA works on (factor_scale_exponents)
 };
 
 // doubles of per-CTA small state: Gc (n+2), Gs 2(n+2), stage (complex: 2(4+3(p-1)); real double
@@ -517,7 +519,12 @@ __device__ __noinline__ void chase_double(const GCtx<double>& cx, int j, Rot2 gi
 
 // Scaled product of the KxK (K = 2 or 3) diagonal blocks at rows/cols i0..i0+K-1 of the
 // triangular factors: Tm 2^e = prod_{l=2..p} H_l[blk]^{s_l} (upper triangular).  A zero
-// diagonal of an inverted factor gives sing = true.
+// diagonal of an inverted factor gives sing = true.  A direct block enters as U 2^ku with the largest
+// entry of U in [0.5, 1); an inverted one entry by entry, split into mantissa and exponent (all
+// exact), so that subnormal or near-overflow entries neither overflow nor lose bits; in the normal
+// range the result is the same, bit for bit.
+constexpr int kNoExp = -(1 << 30);  // exponent of a zero entry
+
 template <int K>
 PSD_DEV void tri_block_product(const GCtx<double>& cx, int i0, double (&Tm)[K][K], int& e, bool& sing) {
   const int p = cx.p, ld = cx.ldh;
@@ -536,6 +543,18 @@ PSD_DEV void tri_block_product(const GCtx<double>& cx, int i0, double (&Tm)[K][K
       for (int c = 0; c < K; c++) U[r][c] = (c >= r) ? PSD_GE(Hl, ld, i0 + r, i0 + c) : 0.0;
     double N[K][K];
     if (cx.Sg(l)) {
+      double mu = 0.0;
+#pragma unroll
+      for (int r = 0; r < K; r++)
+#pragma unroll
+        for (int c = 0; c < K; c++) mu = fmax(mu, fabs(U[r][c]));
+      int ku = 0;
+      if (mu > 0.0 && isfinite(mu)) (void)frexp(mu, &ku);
+#pragma unroll
+      for (int r = 0; r < K; r++)
+#pragma unroll
+        for (int c = 0; c < K; c++) U[r][c] = scalbn(U[r][c], -ku);
+      e += ku;
       // N = Tm * U
 #pragma unroll
       for (int r = 0; r < K; r++)
@@ -548,26 +567,57 @@ PSD_DEV void tri_block_product(const GCtx<double>& cx, int i0, double (&Tm)[K][K
           N[r][c] = acc;
         }
     } else {
-      // N = Tm * inv(U): solve N U = Tm row by row (forward substitution over columns)
+      // N = Tm * inv(U): solve N U = Tm row by row (forward substitution over columns), with one
+      // exponent per entry, N = q 2^x: a quotient by a diagonal entry far below the rest of the block
+      // (a subnormal one) leaves the double range before the block is rescaled.  Each entry's terms
+      // are summed at the exponent of the largest; every division is by a mantissa (pow2_split).
+      double q[K][K];
+      int x[K][K];
+      int ex = kNoExp;
 #pragma unroll
       for (int r = 0; r < K; r++)
 #pragma unroll
         for (int c = 0; c < K; c++) {
-          if (c < r) {
-            N[r][c] = 0.0;
-            continue;
+          q[r][c] = 0.0;
+          x[r][c] = 0;
+          if (c < r) continue;
+          int xm = (Tm[r][c] != 0.0) ? 0 : kNoExp;
+          double um[K];
+          int ue[K];
+#pragma unroll
+          for (int k = 0; k < K; k++) {
+            um[k] = pow2_split(U[k][c], ue[k]);
+            if (k >= r && k < c && q[r][k] != 0.0 && U[k][c] != 0.0) xm = max(xm, x[r][k] + ue[k]);
           }
-          double acc = Tm[r][c];
+          if (xm == kNoExp) xm = 0;
+          double acc = scalbn(Tm[r][c], -xm);
 #pragma unroll
           for (int k = 0; k < K; k++)
-            if (k >= r && k < c) acc = fma(-N[r][k], U[k][c], acc);
+            if (k >= r && k < c)  // (a zero term keeps its sign but not its exponent, which can be huge)
+              acc = fma(-q[r][k], scalbn(um[k], (q[r][k] != 0.0 && um[k] != 0.0) ? x[r][k] + ue[k] - xm : 0), acc);
           if (U[c][c] == 0.0) {
             sing = true;
-            N[r][c] = acc;
+            q[r][c] = acc;
+            x[r][c] = xm;
           } else {
-            N[r][c] = acc / U[c][c];
+            int kd;
+            const double md = pow2_split(U[c][c], kd);
+            q[r][c] = acc / md;
+            x[r][c] = xm - kd;
+          }
+          if (q[r][c] != 0.0 && isfinite(q[r][c])) {
+            int eq;
+            (void)frexp(q[r][c], &eq);
+            ex = max(ex, eq + x[r][c]);
           }
         }
+      if (ex == kNoExp) ex = 0;
+#pragma unroll
+      for (int r = 0; r < K; r++)
+#pragma unroll
+        for (int c = 0; c < K; c++) Tm[r][c] = scalbn(q[r][c], x[r][c] - ex);
+      e += ex;
+      continue;
     }
     double m = 0.0;
 #pragma unroll
@@ -1514,6 +1564,64 @@ PSD_DEV int gpqz_cta(const GCtx<T>& cx, const GqState<T>& st, bool wantT, int ma
 }
 
 
+// Factors whose largest entry lies outside [2^-500, 2^500] are scaled by an exact power of two into
+// [0.5, 1) before the reduction: the QZ's absolute thresholds (safmin / ulp) take an inverted factor
+// near 1e-300 for a singular one, and subnormal or near-overflow factors do not converge.  ex[l-1]
+// receives the exponent e_l (factor l was multiplied by 2^-e_l; 0: left as it was) and the return
+// value is the shift of the eigenvalues, sum over l of s_l ? e_l : -e_l.  Factors inside the window
+// are not touched, so results on them are the same bit for bit.  All threads of the CTA call this;
+// `cell` is one word of shared memory for the reduction.
+template <class T>
+__device__ __noinline__ long long factor_scale_exponents(const GCtx<T>& cx, int* ex, long long* cell) {
+  const int n = cx.n, p = cx.p, tid = cx.tid, nt = cx.nt;
+  long long shift = 0;
+  for (int l = 1; l <= p; l++) {
+    T* Hl = cx.Hp(l);
+    double m = 0.0;
+    for (int e = tid; e < n * n; e += nt) m = fmax(m, fmax(fabs(re_(Hl[(e % n) + (size_t)(e / n) * cx.ldh])),
+                                                           fabs(im_(Hl[(e % n) + (size_t)(e / n) * cx.ldh]))));
+    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if (tid == 0) *cell = 0;
+    __syncthreads();
+    // the bit patterns of non-negative doubles order as the values do
+    if ((tid & 31) == 0) atomicMax(cell, __double_as_longlong(m));
+    __syncthreads();
+    m = __longlong_as_double(*cell);
+    __syncthreads();
+    int k = 0;
+    if (m > 0.0 && isfinite(m) && (m < 0x1p-500 || m > 0x1p500)) (void)frexp(m, &k);
+    if (k != 0)
+      for (int e = tid; e < n * n; e += nt) {
+        T& x = Hl[(e % n) + (size_t)(e / n) * cx.ldh];
+        x = scal2(x, -k);
+      }
+    if (tid == 0) ex[l - 1] = k;
+    shift += cx.Sg(l) ? k : -k;
+  }
+  __syncthreads();
+  return shift;
+}
+
+// Undoes factor_scale_exponents: the eigenvalues (finite, non-zero; al == nullptr: none) by
+// 2^eshift, factor l of T by 2^e_l.
+template <class T>
+__device__ __noinline__ void undo_factor_scale(const GCtx<T>& cx, const int* ex, long long eshift, const cplx* al,
+                                               const T* be, long long* sc) {
+  const int n = cx.n, tid = cx.tid, nt = cx.nt;
+  if (al && eshift != 0)
+    for (int i = tid; i < n; i += nt)
+      if (!is_zero(be[i]) && !(al[i].x == 0.0 && al[i].y == 0.0)) sc[i] += eshift;
+  for (int l = 1; l <= cx.p; l++) {
+    const int k = ex[l - 1];
+    if (k == 0) continue;
+    T* Hl = cx.Hp(l);
+    for (int e = tid; e < n * n; e += nt) {
+      T& x = Hl[(e % n) + (size_t)(e / n) * cx.ldh];
+      x = scal2(x, k);
+    }
+  }
+}
+
 template <class T, int MAXT>
 __global__ void __launch_bounds__(MAXT, 1) gpschur_kernel(GpqzParams<T> P) {
   const int n = P.n, p = P.p, tid = threadIdx.x, nt = blockDim.x;
@@ -1584,6 +1692,8 @@ __global__ void __launch_bounds__(MAXT, 1) gpschur_kernel(GpqzParams<T> P) {
     }
     __syncthreads();
 
+    int* ex = P.pexp + (size_t)blockIdx.x * p;
+    const long long eshift = factor_scale_exponents(cx, ex, &s_b);  // (s_b is free until the next problem)
     const long long tstart = clock64();
     if (!P.skip_reduce) {
       gphessenberg_cta(cx);
@@ -1616,6 +1726,8 @@ __global__ void __launch_bounds__(MAXT, 1) gpschur_kernel(GpqzParams<T> P) {
       printf("[psd gpschur b=%lld] stage1 %lld  stage2 %lld  qz %lld cycles\n", b,
              P.skip_reduce ? 0LL : s_prof[0] - tstart, P.skip_reduce ? 0LL : tred - s_prof[0], clock64() - tred);
     if (tid == 0) P.info[b] = info;
+    __syncthreads();
+    undo_factor_scale(cx, ex, eshift, P.reduce_only ? nullptr : al, be, sc);
     __syncthreads();
 
     if (P.use_smem) {

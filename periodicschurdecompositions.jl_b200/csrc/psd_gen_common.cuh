@@ -56,6 +56,8 @@ PSD_DEV double abs_(cplx a) { return hypot(a.x, a.y); }
 PSD_DEV double abs_(double a) { return fabs(a); }
 PSD_DEV double abs1_(cplx a) { return fabs(a.x) + fabs(a.y); }
 PSD_DEV bool is_zero(cplx a) { return a.x == 0.0 && a.y == 0.0; }
+PSD_DEV cplx scal2(cplx a, int k) { return mk(scalbn(a.x, k), scalbn(a.y, k)); }
+PSD_DEV double scal2(double a, int k) { return scalbn(a, k); }
 PSD_DEV bool is_zero(double a) { return a == 0.0; }
 // Smith's complex division
 PSD_DEV cplx operator/(cplx a, cplx b) {
@@ -1394,8 +1396,27 @@ PSD_DEV void gphessenberg_cta(const GCtx<T>& cx) {
   }
 }
 
+// x = m 2^k exactly, with the larger of |Re m|, |Im m| in [0.5, 1); m = x and k = 0 for a zero.
+// Products of diagonal entries multiply (divide) mantissas and add (subtract) exponents: the raw
+// product overflows above about 9e307, a quotient by a subnormal overflows, and a product with a
+// subnormal rounds onto the subnormal grid.  In the normal range the result is the same, bit for bit.
+PSD_DEV double pow2_split(double x, int& k) {
+  k = 0;
+  if (x == 0.0 || !isfinite(x)) return x;
+  (void)frexp(x, &k);
+  return scalbn(x, -k);
+}
+PSD_DEV cplx pow2_split(cplx x, int& k) {
+  k = 0;
+  const double big = fmax(fabs(x.x), fabs(x.y));
+  if (big == 0.0 || !isfinite(big)) return x;
+  (void)frexp(big, &k);
+  return mk(scalbn(x.x, -k), scalbn(x.y, -k));
+}
+
 // generalized.jl:939-976 (_safeprod): x_1^{s_1} prod x_l^{s_l} = alpha / beta * 2^scale with
-// |alpha| in [1,2) or 0 and beta in {0,1}.  d[l-1] = diagonal entry of factor l.
+// |alpha| in [1,2) or 0 and beta in {0,1}.  d[l-1] = diagonal entry of factor l.  Unlike the
+// reference, each x_l enters split into mantissa and exponent (pow2_split).
 template <class T, class F>
 PSD_DEV void safeprod(int p, const unsigned char* S, F diag_of, T& alpha, int& beta, long long& scale) {
   alpha = Scalar<T>::one();
@@ -1403,13 +1424,18 @@ PSD_DEV void safeprod(int p, const unsigned char* S, F diag_of, T& alpha, int& b
   scale = 0;
   for (int i = 1; i <= p; i++) {
     const T xi = diag_of(i);
+    int k;
+    const T mi = pow2_split(xi, k);
     if (S[i - 1]) {
-      alpha = alpha * xi;
+      alpha = alpha * mi;
+      scale += k;
     } else {
-      if (is_zero(xi))
+      if (is_zero(xi)) {
         beta = 0;
-      else
-        alpha = alpha / xi;
+      } else {
+        alpha = alpha / mi;
+        scale -= k;
+      }
     }
     double aa = abs_(alpha);
     if (aa == 0.0) {
