@@ -307,6 +307,45 @@ int psd_rcheckpsd_batched(psd_handle_t handle, int n, int p, int64_t batch, int 
                           const double* A, const double* T, const double* Z, double* err,
                           double* tri, double* orth);
 
+/* Eigenvectors of real periodic Schur decompositions, batched.
+ * Replaces eigvecs(P::PeriodicSchur) of the reference for S all true.  The reference moves each
+ * eigenvalue to the top with ordschur! and reads the vectors off the reordered Z; here they come
+ * from a periodic back-substitution on the Schur form (the analogue of LAPACK trevc for a product
+ * of triangular factors), with no reordering.
+ *   T       in  [batch][p][n][n]  the T factors of psd_rpschur_batched (wantT), user order
+ *   Z       in  [batch][p][n][n]  the Z factors of the same call
+ *   select  in  [batch][n] (nonzero = wanted) or NULL for every eigenvalue
+ *   V       out [batch][p][n][n] complex128: column k of V_l is v_l for eigenvalue eig[k],
+ *                                   with  :R  A_l v_{l+1} = mu_l v_l,  :L  A_l v_l = mu_l v_{l+1}
+ *                                   (v_{p+1} = v_1) and prod_l mu_l = eig[k]
+ *   info    out [batch]: 0 = success, 1 = T is not in periodic Schur form (two adjacent nonzero
+ *                        subdiagonal entries of the Schur factor, a nonzero subdiagonal entry of
+ *                        another factor, or a 2x2 block whose product has real eigenvalues); that
+ *                        problem's V is zero.  2 = a selected vector came out zero or not finite
+ *                        (non-finite input): its columns are zero, the other columns are valid.
+ *                        One bad problem never fails the batch.
+ * Every vector has unit 2-norm and its entry of largest modulus (lowest row on ties) is real and
+ * positive; columns not selected are exactly zero.  A real eigenvalue gives a vector with zero
+ * imaginary parts.  A complex pair at (k, k+1) (exactly nonzero subdiagonal of the Schur factor,
+ * eig[k] with positive imaginary part first) fills both columns when either is selected, column
+ * k+1 being the exact conjugate of column k.  Of the entries below the (quasi-)triangle of T only
+ * the first subdiagonal is read (2x2 blocks, structure check); the others are never read.
+ * Below n = 192 each column is computed by its own warp and CTA-level product, so its bits do not
+ * depend on which other columns are selected.  n >= 192: the back-transformation V_l = Z_l X_l runs
+ * on the FP64 tensor-core GEMM, one problem at a time; with few vectors that GEMM splits K and adds
+ * the parts with floating-point atomics, so these results are not bit-for-bit reproducible from run
+ * to run nor independent of the selection (every stated property holds). */
+int psd_reigvecs_batched(psd_handle_t handle, int n, int p, int64_t batch, int orientation,
+                         const double* T, const double* Z, const uint8_t* select, double* V,
+                         int32_t* info);
+
+/* The same for complex results: T and Z complex128 [batch][p][n][n], the complex standard result
+ * of psd_cpschur_batched with S all true (upper triangular T; any nonzero subdiagonal entry gives
+ * info = 1).  Replaces eigvecs(P::PeriodicSchur) for ComplexF64 factors. */
+int psd_ceigvecs_batched(psd_handle_t handle, int n, int p, int64_t batch, int orientation,
+                         const double* T, const double* Z, const uint8_t* select, double* V,
+                         int32_t* info);
+
 #ifdef __cplusplus
 }
 #endif

@@ -39,6 +39,8 @@ from .pschur import (  # noqa: F401
     pschur_batched,
     pschur_hessut_batched,
     checkpsd_batched,
+    eigvecs,
+    eigvecs_batched,
     phessenberg_packed_batched,
     shard_bounds,
 )
@@ -46,5 +48,5 @@ from .pschur import (  # noqa: F401
 __all__ = [
     "PsdError", "device_count", "lib", "lib_path", "library_available", "version",
     "PeriodicSchur", "GeneralizedPeriodicSchur", "gpschur", "gpschur_", "gpschur_batched", "gphessenberg_batched", "gvalues", "Handle", "default_handle", "phessenberg_batched", "rphessenberg_rowwise_batched", "pschur", "pschur_",
-    "pschur_batched", "pschur_hessut_batched", "checkpsd_batched", "phessenberg_packed_batched", "shard_bounds",
+    "pschur_batched", "pschur_hessut_batched", "checkpsd_batched", "eigvecs", "eigvecs_batched", "phessenberg_packed_batched", "shard_bounds",
 ]

@@ -38,6 +38,8 @@ EXPORTED_SYMBOLS = [
     "psd_host_alloc",
     "psd_host_free",
     "psd_rcheckpsd_batched",
+    "psd_reigvecs_batched",
+    "psd_ceigvecs_batched",
     "psd_fill_uniform_host",
     "psd_fill_uniform_dev",
 ]
@@ -88,6 +90,8 @@ def lib():
         L.psd_host_free.argtypes = [vp]
         L.psd_rphess_packed_batched.argtypes = [vp, C.c_int, C.c_int, C.c_int64, vp, vp]
         L.psd_rcheckpsd_batched.argtypes = [vp, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp, vp, vp, vp, vp]
+        L.psd_reigvecs_batched.argtypes = [vp, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp, vp, vp, vp]
+        L.psd_ceigvecs_batched.argtypes = L.psd_reigvecs_batched.argtypes
         L.psd_rphess_batched.argtypes = [vp, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp]
         L.psd_cpschur_batched.argtypes = [vp, C.c_int, C.c_int, C.c_int64, C.c_int, vp, C.c_int,
                                           C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]

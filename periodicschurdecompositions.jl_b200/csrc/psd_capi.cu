@@ -21,6 +21,7 @@
 #include "../../include/psd_b200.h"
 #include "psd_real_kernel.cuh"
 #include "psd_checkpsd.cuh"
+#include "psd_eigvecs.cuh"
 #include "psd_real_hess32.cuh"
 #include "psd_cplx_qz.cuh"
 #include "psd_rowhess.cuh"
@@ -59,8 +60,9 @@ int fail(int code, const std::string& msg) {
 constexpr int kSlotsPerDevice = 3;
 
 // Roles of the pipeline buffers of a batched host call: the factors (A in, T out), Z, the
-// eigenvalues (real: eig in kVal0; generalized: alpha, beta, alphascale), info, iteration counts.
-enum Role { kFactors, kZ, kVal0, kVal1, kVal2, kInfo, kIters, kRoles };
+// eigenvalues (real: eig in kVal0; generalized: alpha, beta, alphascale), info, iteration counts;
+// the eigenvector calls add their slot columns and the vectors V.
+enum Role { kFactors, kZ, kVal0, kVal1, kVal2, kInfo, kIters, kCols, kVecs, kRoles };
 
 struct Slot {
   cudaStream_t stream = nullptr;
@@ -1056,6 +1058,168 @@ int run_gen_host(psd_handle_t h, const GenCall& gc, int64_t batch, void* A, void
   });
 }
 
+// ---------------------------------------------------------------------------------------------
+// Eigenvectors of periodic Schur results by periodic back-substitution (psd_eigvecs.cuh).
+// ---------------------------------------------------------------------------------------------
+struct EigvecCall {
+  int n, p, left, cplx;
+};
+
+// Slots of every problem, in column order: each selected column, and a complex pair (exactly
+// nonzero subdiagonal of the Schur factor, as the reference detects its 2x2 blocks) once, at its
+// first column, when either member is selected.  cols[b][slot] = column, -1 after the last slot;
+// rows[b] = 1 + the top row of the last slot (the rows of X that can be nonzero).
+void plan_eigvec_slots(const EigvecCall& ec, int64_t batch, const double* T, const uint8_t* select,
+                       std::vector<int32_t>& cols, std::vector<int>& count, std::vector<int>& rows) {
+  const int n = ec.n, p = ec.p;
+  const size_t nn = (size_t)n * n, es = ec.cplx ? 2 : 1;
+  cols.assign((size_t)batch * n, -1);
+  count.assign((size_t)batch, 0);
+  rows.assign((size_t)batch, 0);
+  for (int64_t b = 0; b < batch; b++) {
+    const double* T1 = T + ((size_t)b * p + (ec.left ? p - 1 : 0)) * nn * es;
+    const uint8_t* sel = select ? select + (size_t)b * n : nullptr;
+    int m = 0;
+    for (int c = 0; c < n; c++) {
+      const bool pair = !ec.cplx && c + 1 < n && T1[(c + 1) + (size_t)c * n] != 0.0;
+      if (!sel || sel[c] || (pair && sel[c + 1])) {
+        cols[(size_t)b * n + m++] = c;
+        rows[b] = c + (pair ? 2 : 1);
+      }
+      if (pair) c++;
+    }
+    count[b] = m;
+  }
+}
+
+// Enqueues the eigenvectors of problems first .. first+nb-1 (device buffers d[role] of the chunk).
+int launch_eigvecs(psd_handle_s* h, Device& dev, Slot& s, const EigvecCall& ec, long long first, long long nb,
+                   const std::vector<int>& count, const std::vector<int>& rows, void* const* d) {
+  const int n = ec.n, p = ec.p;
+  const size_t nn = (size_t)n * n, es = ec.cplx ? 16 : 8;
+  const cudaStream_t st = s.stream;
+  PSD_CUDA(cudaMemsetAsync(d[kVecs], 0, (size_t)nb * p * nn * 16, st));
+  PSD_CUDA(cudaMemsetAsync(d[kInfo], 0, (size_t)nb * sizeof(int32_t), st));
+  void (*prep)(psd::EigvecParams) = ec.cplx ? psd::eigvecs_prep_kernel<psd::cplx> : psd::eigvecs_prep_kernel<double>;
+  void (*kern)(psd::EigvecParams) = ec.cplx ? psd::eigvecs_kernel<psd::cplx> : psd::eigvecs_kernel<double>;
+  void (*fin)(psd::EigvecParams, const double*) =
+      ec.cplx ? psd::eigvecs_finish_kernel<psd::cplx> : psd::eigvecs_finish_kernel<double>;
+  int optin = 0;
+  PSD_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev.ordinal));
+  cudaFuncAttributes fa;
+  PSD_CUDA(cudaFuncGetAttributes(&fa, kern));
+  const size_t max_dyn = (size_t)optin - fa.sharedSizeBytes;
+  // factor scales and exponents, staging of the solved rows; then per slot [ws, x, s] in shared
+  // memory, or in global memory from the large-N threshold on (and wherever they do not fit)
+  const size_t head = (size_t)((p + 1) & ~1) * sizeof(double) + (size_t)psd::EV_CB * p * 2 * 16;
+  const size_t full = head + (size_t)psd::EV_CB * p * (psd::EV_WS + 2 * (size_t)n) * 16;
+  const bool global = n >= kLargeN || full > max_dyn;
+  PSD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(global ? head : full)));
+  psd::EigvecParams P;
+  P.n = n; P.p = p; P.left = ec.left;
+  P.X = nullptr; P.S = nullptr; P.W = nullptr;
+  if (int e = ensure_dev(s.dPexp, s.capPexp, (size_t)nb * p * sizeof(int))) return e;
+  P.fexp = s.dPexp;
+  ScopedKernelTimer tm(h, dev, st, 1);
+  if (!global) {
+    int mmax = 0;
+    for (long long b = first; b < first + nb; b++) mmax = std::max(mmax, count[b]);
+    P.nblk = std::max(1, (mmax + psd::EV_CB - 1) / psd::EV_CB);
+    P.batch = nb;
+    P.T = d[kFactors]; P.Z = d[kZ]; P.cols = (const int*)d[kCols]; P.info = (int32_t*)d[kInfo];
+    P.V = (psd::cplx*)d[kVecs];
+    P.global_mode = 0; P.m = 0;
+    const int threads = (p * n > 128) ? 256 : 128;
+    prep<<<dim3((unsigned)nb, (unsigned)p), 256, 0, st>>>(P);
+    kern<<<(unsigned)(nb * P.nblk), threads, full, st>>>(P);
+    PSD_CUDA(cudaGetLastError());
+    __atomic_fetch_add(&h->stats[0], (int64_t)2, __ATOMIC_RELAXED);
+    __atomic_fetch_add(&h->stats[1], (int64_t)nb, __ATOMIC_RELAXED);
+    return PSD_OK;
+  }
+  for (long long bi = 0; bi < nb; bi++) {
+    const int m = count[first + bi];
+    const size_t vec = (size_t)std::max(m, 1) * p * n;  // complex entries of X (and of S)
+    int e = ensure_dev(s.dScratch, s.capScratch,
+                       (2 * vec * 2 + (size_t)std::max(m, 1) * p * psd::EV_WS * 2 + 2 * vec) * sizeof(double));
+    if (e) return e;
+    P.X = (psd::cplx*)s.dScratch;
+    P.S = P.X + vec;
+    P.W = P.S + vec;
+    double* Wv = (double*)(P.W + (size_t)std::max(m, 1) * p * psd::EV_WS);  // [re, im][p][m][n]
+    P.nblk = std::max(1, (m + psd::EV_CB - 1) / psd::EV_CB);
+    P.batch = 1;
+    P.T = (const char*)d[kFactors] + bi * p * nn * es;
+    P.Z = (const char*)d[kZ] + bi * p * nn * es;
+    P.cols = (const int*)d[kCols] + bi * n;
+    P.info = (int32_t*)d[kInfo] + bi;
+    P.V = (psd::cplx*)d[kVecs] + bi * p * nn;
+    P.global_mode = 1; P.m = m;
+    P.fexp = s.dPexp + bi * p;
+    prep<<<dim3(1, (unsigned)p), 256, 0, st>>>(P);
+    kern<<<P.nblk, 256, head, st>>>(P);
+    PSD_CUDA(cudaGetLastError());
+    if (m == 0) continue;
+    // V_u = Z_u X_u over the rows of X that can be nonzero: a real Z times a complex X is two
+    // real products, a complex Z four
+    const int K = rows[first + bi];
+    for (int u = 0; u < p; u++) {
+      const double* Zu = (const double*)P.Z + (size_t)u * nn * (es / 8);
+      const double* Xu = (const double*)(P.X + (size_t)u * m * n);
+      auto gemm = [&](int zpart, int xpart, int wpart, double alpha, double beta) -> cudaError_t {
+        psd::GemmArgs g;
+        g.M = n; g.N = m; g.K = K;
+        g.A = Zu + zpart; g.rsA = ec.cplx ? 2 : 1; g.csA = (long long)n * (ec.cplx ? 2 : 1);
+        g.B = Xu + xpart; g.rsB = 2; g.csB = 2LL * n;
+        g.C = Wv + ((size_t)wpart * p + u) * m * n; g.ldc = n;
+        g.alpha = alpha; g.beta = beta; g.splitK = 1;
+        return psd::dgemm_launch(st, dev.sm_count, g);
+      };
+      PSD_CUDA(gemm(0, 0, 0, 1.0, 0.0));
+      PSD_CUDA(gemm(0, 1, 1, 1.0, 0.0));
+      if (ec.cplx) {
+        PSD_CUDA(gemm(1, 1, 0, -1.0, 1.0));
+        PSD_CUDA(gemm(1, 0, 1, 1.0, 1.0));
+      }
+    }
+    fin<<<(unsigned)((m * p + 3) / 4), 128, 0, st>>>(P, Wv);
+    PSD_CUDA(cudaGetLastError());
+    __atomic_fetch_add(&h->stats[0], (int64_t)(3 + p * (ec.cplx ? 4 : 2)), __ATOMIC_RELAXED);
+  }
+  __atomic_fetch_add(&h->stats[2], (int64_t)nb, __ATOMIC_RELAXED);
+  return PSD_OK;
+}
+
+int run_eigvecs_host(psd_handle_t h, const EigvecCall& ec, int64_t batch, const double* T, const double* Z,
+                     const uint8_t* select, double* V, int32_t* info) {
+  if (ec.n < 1 || ec.p < 1 || batch < 0) return fail(PSD_ERR_BAD_ARG, "n, p must be >= 1 and batch >= 0");
+  if (ec.left != 0 && ec.left != 1)
+    return fail(PSD_ERR_BAD_ARG, "orientation argument must be either 0 (:R, right) or 1 (:L, left)");
+  if (!T || !Z || !V || !info) return fail(PSD_ERR_BAD_ARG, "T, Z, V and info must not be NULL");
+  if (!h) return fail(PSD_ERR_BAD_ARG, "null handle");
+  if (h->devs.empty()) return fail(PSD_ERR_NO_DEVICE, "handle has no CUDA device");
+  std::vector<int32_t> cols;
+  std::vector<int> count, rows;
+  plan_eigvec_slots(ec, batch, T, select, cols, count, rows);
+  const size_t nn = (size_t)ec.n * ec.n;
+  const size_t per = nn * ec.p * (ec.cplx ? 16 : 8);  // bytes of T (and of Z) per problem
+  const size_t perV = nn * ec.p * 16;
+  return run_host(h, batch, {T, Z, V, info}, [&](Device& dev, long long first, long long count_d, bool pinned,
+                                                 int64_t* bytes_h2d, int64_t* bytes_d2h) {
+    std::vector<HostArray> in{{(char*)T, per, kFactors}, {(char*)Z, per, kZ},
+                              {(char*)cols.data(), ec.n * sizeof(int32_t), kCols, false}};
+    std::vector<HostArray> out{{(char*)V, perV, kVecs}, {(char*)info, sizeof(int32_t), kInfo}};
+    long long off = first;  // run_shard launches the chunks in order
+    auto launch = [&](Slot& s, long long nb, void* const* d) {
+      const int e = launch_eigvecs(h, dev, s, ec, off, nb, count, rows, d);
+      off += nb;
+      return e;
+    };
+    return run_shard(dev, first, plan_real_chunks(count_d, 2 * per + perV, pinned), pinned, in, out, launch,
+                     bytes_h2d, bytes_d2h);
+  });
+}
+
 }  // namespace
 
 extern "C" {
@@ -1238,6 +1402,16 @@ int psd_rcheckpsd_batched(psd_handle_t h, int n, int p, int64_t batch, int orien
 #undef PSD_CHK
   cleanup();
   return PSD_OK;
+}
+
+int psd_reigvecs_batched(psd_handle_t h, int n, int p, int64_t batch, int orientation, const double* T,
+                         const double* Z, const uint8_t* select, double* V, int32_t* info) {
+  return run_eigvecs_host(h, EigvecCall{n, p, orientation, 0}, batch, T, Z, select, V, info);
+}
+
+int psd_ceigvecs_batched(psd_handle_t h, int n, int p, int64_t batch, int orientation, const double* T,
+                         const double* Z, const uint8_t* select, double* V, int32_t* info) {
+  return run_eigvecs_host(h, EigvecCall{n, p, orientation, 1}, batch, T, Z, select, V, info);
 }
 
 int psd_rphess_packed_batched(psd_handle_t h, int n, int p, int64_t batch, double* A, double* tau) {

@@ -278,4 +278,49 @@ function phessenberg!(A::Vector{Matrix{Float64}}; handle::Handle = default_handl
     return H1, pH
 end
 
+# ---- eigenvectors of PeriodicSchur results (psd_reigvecs_batched / psd_ceigvecs_batched) -------
+"""
+    eigvecs_batched(T, Z, lr = :R; select = nothing, handle) -> (V, info)
+
+Eigenvectors of `batch` periodic Schur results at once, by periodic back-substitution on the Schur
+form.  `T` and `Z` are `(n, n, p, batch)` arrays of `Float64` or `ComplexF64` in user factor order
+(the layout `pschur!` packs for the device); `select` an `(n, batch)` `Bool` array or `nothing`
+for every eigenvalue.  `V[:, k, l, b]` is the unit vector `v_l` of eigenvalue `k` of problem `b`
+(`:R`: `A_l v_{l+1} = mu_l v_l`, `:L`: `A_l v_l = mu_l v_{l+1}`, `prod(mu) = values[k]`), with its
+entry of largest modulus real and positive; unselected columns are zero and a complex pair is
+filled whole when either member is selected.  `info[b] == 1`: `T` of problem `b` is not in periodic
+Schur form.
+
+This is deliberately the module's own function and not a method of `LinearAlgebra.eigvecs` for the
+reference's structs: the reference computes its vectors by reordering with `ordschur!`, and the
+normalisation and layout of its return value cannot be confirmed here.  Like the rest of this file
+the glue has not been executed; the same ABI is exercised by the Python mirror (`../pschur.py`).
+"""
+function eigvecs_batched(T::Array{E, 4}, Z::Array{E, 4}, lr::Symbol = :R;
+                         select::Union{Nothing, AbstractMatrix{Bool}} = nothing,
+                         handle::Handle = default_handle()) where {E <: Union{Float64, ComplexF64}}
+    o = orient_code(lr)
+    n, n2, p, batch = size(T)
+    (n == n2 && size(Z) == size(T)) || throw(DimensionMismatch("T and Z must be (n, n, p, batch)"))
+    sel = select === nothing ? C_NULL : convert(Array{UInt8}, select)
+    select === nothing || size(select) == (n, batch) || throw(DimensionMismatch("select must be (n, batch)"))
+    V = zeros(ComplexF64, n, n, p, batch)
+    info = zeros(Int32, batch)
+    rc = GC.@preserve sel begin
+        if E === Float64
+            ccall((:psd_reigvecs_batched, libpsd), Cint,
+                  (Ptr{Cvoid}, Cint, Cint, Int64, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8},
+                   Ptr{ComplexF64}, Ptr{Int32}),
+                  handle.ptr, n, p, batch, o, T, Z, sel, V, info)
+        else
+            ccall((:psd_ceigvecs_batched, libpsd), Cint,
+                  (Ptr{Cvoid}, Cint, Cint, Int64, Cint, Ptr{ComplexF64}, Ptr{ComplexF64}, Ptr{UInt8},
+                   Ptr{ComplexF64}, Ptr{Int32}),
+                  handle.ptr, n, p, batch, o, T, Z, sel, V, info)
+        end
+    end
+    rc == 0 || error(lasterror(rc))
+    return V, info
+end
+
 end # module

@@ -222,6 +222,68 @@ def checkpsd_batched(A: np.ndarray, T: np.ndarray, Z: np.ndarray, lr="R", thresh
     return ok, err, tri, orth
 
 
+def eigvecs_batched(T: np.ndarray, Z: np.ndarray, lr="R", select=None, handle: Optional[Handle] = None):
+    """Eigenvectors of batched periodic Schur results (psd_reigvecs_batched for float64 T and Z,
+    psd_ceigvecs_batched for complex128), by periodic back-substitution on the Schur form.
+
+    T, Z: [batch][p][n][n] storage layout, user factor order, as pschur_batched / gpschur_batched
+    (S all true) return them.  select: [batch][n] (or [n] for every problem) booleans, None = all.
+    Returns (V, info): V complex128 [batch][p][n][n] with column k of V[b, l] the unit vector v_l of
+    eigenvalue k (zero where not selected), info int32 [batch] (1 = T not in periodic Schur form)."""
+    orient = char_lr(lr)
+    if T.ndim != 4 or T.shape[2] != T.shape[3] or T.shape != Z.shape or T.dtype != Z.dtype \
+            or T.dtype not in (np.float64, np.complex128):
+        raise ValueError("T and Z must be float64 or complex128 with equal shape [batch][p][n][n]")
+    h = handle or default_handle()
+    batch, p, n, _ = T.shape
+    T = np.ascontiguousarray(T)
+    Z = np.ascontiguousarray(Z)
+    sel = None
+    if select is not None:
+        sel = np.ascontiguousarray(np.broadcast_to(np.asarray(select, dtype=bool), (batch, n)).astype(np.uint8))
+    V = np.empty((batch, p, n, n), dtype=np.complex128)
+    info = np.empty(batch, dtype=np.int32)
+    f = lib().psd_ceigvecs_batched if T.dtype == np.complex128 else lib().psd_reigvecs_batched
+    check(f(h.ptr, n, p, batch, 1 if orient == "L" else 0, _vp(T), _vp(Z), _vp(sel), _vp(V), _vp(info)))
+    return V, info
+
+
+def eigvecs(P: PeriodicSchur, select=None, handle: Optional[Handle] = None) -> List[np.ndarray]:
+    """Eigenvectors of a PeriodicSchur result: p matrices (n x m, math orientation), matrix l holding
+    v_l of every selected eigenvalue (all when select is None) in eigenvalue order; a complex pair
+    is kept whole when either member is selected.  :R  A_l v_{l+1} = mu_l v_l,
+    :L  A_l v_l = mu_l v_{l+1}, prod mu_l = values[k]."""
+    p = P.period
+    n = P.T1.shape[0]
+    if len(P.Z) != p or P.Z[0].shape != (n, n):
+        raise ValueError("eigvecs needs the Schur vectors (pschur with wantZ)")
+    dt = np.complex128 if np.iscomplexobj(P.T1) else np.float64
+    Ts = [P.T1] + list(P.T) if P.orientation == "R" else list(P.T) + [P.T1]
+    T = np.empty((1, p, n, n), dtype=dt)
+    Z = np.empty((1, p, n, n), dtype=dt)
+    for j in range(p):
+        T[0, j] = Ts[j].T
+        Z[0, j] = P.Z[j].T
+    V, info = eigvecs_batched(T, Z, P.orientation, None if select is None else np.asarray(select, bool)[None],
+                              handle)
+    if info[0] == 1:
+        raise ValueError("the factors are not in periodic Schur form")
+    if info[0] == 2:
+        raise FloatingPointError("an eigenvector came out zero or not finite")
+    # the columns the library fills: the selected ones, and a complex pair (exactly nonzero
+    # subdiagonal of the Schur factor) whole when either member is selected
+    keep = np.zeros(n, dtype=bool) if select is not None else np.ones(n, dtype=bool)
+    if select is not None:
+        sel = np.asarray(select, dtype=bool)
+        c = 0
+        while c < n:
+            pair = dt == np.float64 and c + 1 < n and P.T1[c + 1, c] != 0
+            w = 2 if pair else 1
+            keep[c:c + w] = sel[c:c + w].any()
+            c += w
+    return [np.ascontiguousarray(V[0, l].T[:, keep]) for l in range(p)]
+
+
 def pschur_hessut_batched(H: np.ndarray, wantZ: bool = True, wantT: bool = True, maxitfac: int = 30,
                           handle: Optional[Handle] = None, Q: Optional[np.ndarray] = None):
     """Inner method pschur!(H1, Hs; ...) (PeriodicSchurDecompositions.jl:322) on Hessenberg /
